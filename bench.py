@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (through the C-ABI)
   python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                   # also writes the last timed step's image: compare two builds with it
 
 Workload (default c5 = BASELINE.json configs[4], the configuration the metric is quoted on "at 1/2/4/8 GPUs"): the
 2,005,056-triangle tessellated Cornell box, full path trace (max depth 8), 3840x2160, 64 spp.  One STEP = one pass of
@@ -60,7 +61,14 @@ def parse():
     ap.add_argument("--sah-traverse", type=float, default=0.0, help="SAH node-visit cost (0 = default 1.2)")
     ap.add_argument("--force-width", type=int, default=0, help="force the scene form: 1 FLAT, 4 4-wide, 2 binary (0 = the library's pick)")
     ap.add_argument("--gpu-build", action="store_true", help="build the BVH on the device (LBVH) instead of the host SAH builder")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the image of the last timed step to DIR/image.npy "
+                                                          "(float32 RGBA rows; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times a shard whose size depends on the host)")
+    return args
 
 
 def dist_env():
@@ -166,6 +174,19 @@ def peaks():
         d = json.load(open(path))
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)", float(d.get("sm_max_mhz", 1965.0))
     return 6650.0, "fallback (B200_PROFILING.md)", 1965.0
+
+
+DUMP_PIXELS = 1 << 21  # 32 MiB of float4 rows
+
+
+def dump_outputs(path, image):
+    """Writes `image` ((pixels, 4) float32, the image a caller of the timed path receives) as path/image.npy: whole when it has at most
+    DUMP_PIXELS pixels, else the rows of DUMP_PIXELS pixels drawn once with seed 0 and kept in ascending order -- the same pixels on
+    every run of the workload, so that the files of two builds compare row for row."""
+    os.makedirs(path, exist_ok=True)
+    if len(image) > DUMP_PIXELS:
+        image = image[np.sort(np.random.default_rng(0).choice(len(image), DUMP_PIXELS, replace=False))]
+    np.save(os.path.join(path, "image.npy"), np.ascontiguousarray(image, np.float32))
 
 
 def ncu_traffic(name):
@@ -453,6 +474,10 @@ class Job:
                 "h2d_bytes_per_step": int((self.tris.nbytes + self.mats.nbytes) * self.world),
                 "d2h_bytes_per_step": int(self.npix * (3 if rgb8 else 16)), "host_checksum": checksum, "steps": steps}
 
+    def image(self):
+        """rank 0's image of the last device_timed step, (pixels, 4) float32"""
+        return self.full[0].read(np.float32).reshape(-1, 4)
+
     def close(self):
         self.barrier()
         for b in self.imported:
@@ -493,6 +518,7 @@ def simt_fraction(job, rays_per_s, sm_count, sm_max_mhz):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, __pycache__ included
     args = parse()
     rank, world, local = dist_env()
     if args.impl == "reference":
@@ -524,8 +550,14 @@ def main():
     job = Job(pt, dev, dist, rank, world, args.workload, args, scenes)
     sampler = ClockSampler(local)
     sampler.start()
-    rays_all, ms_total, ms_steps, prof = job.device_timed(args.steps, args.warmup, flush, stream, sampler)
-    clocks = sampler.stop()
+    try:
+        rays_all, ms_total, ms_steps, prof = job.device_timed(args.steps, args.warmup, flush, stream, sampler)
+    finally:
+        clocks = sampler.stop()  # no nvidia-smi left running if the timed steps fail
+    if args.dump_outputs:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, job.image())
+        job.barrier()  # e2e() on every rank renders into rank 0's images
     value = rays_all / (ms_total * 1e-3) / 1e6
     launches = int(prof["kernel_launches"])
     e2e = None

@@ -232,7 +232,7 @@ def test_product_never_imports_oracle():
             assert needle not in src, (f, needle)
 
 
-def test_raycast_host_program_refuses_without_gpu(pt):
+def test_raycast_host_program_refuses_without_gpu(pt, tmp_path):
     """The C++ mirror of DeviceTest.RayCast (host/raycast_main.cpp) exits loudly when there is no device."""
     import subprocess
     exe = os.path.join(ROOT, "oclpathtracer_b200", "host", "ptb_raycast")
@@ -241,7 +241,7 @@ def test_raycast_host_program_refuses_without_gpu(pt):
     n = C.c_int(-1)
     if pt.lib().ptb_device_count(C.byref(n)) == 0 and n.value > 0:
         pytest.skip("a CUDA device is present")
-    r = subprocess.run([exe, SCENE, "/tmp/unused.ppm", "32", "1"], capture_output=True, text=True)
+    r = subprocess.run([exe, SCENE, str(tmp_path / "unused.ppm"), "32", "1"], capture_output=True, text=True)
     assert r.returncode == 2 and "no CUDA device" in r.stderr
 
 
@@ -363,3 +363,21 @@ def test_bench_reference_arm_under_torchrun():
     assert len(os.sched_getaffinity(0)) == 1 or d["cpu_baseline"]["cores"] > 1
     import bench
     assert d["config"] == bench.config_of("c5", 2) and d["config"]["workload"].startswith("c5")  # default workload, same config as our arm
+
+
+def test_bench_dump_outputs_samples_large_images(tmp_path):
+    """bench.py --dump-outputs: an image larger than DUMP_PIXELS is written as the rows of a fixed sample of distinct pixels in
+    ascending order, identical from run to run and far below 64 MB; a smaller one is written whole."""
+    import bench
+    n = bench.DUMP_PIXELS + 1_000_000
+    img = np.arange(n * 4, dtype=np.float32).reshape(n, 4)  # row k holds 4k .. 4k+3, exact in float32
+    bench.dump_outputs(str(tmp_path / "a"), img)
+    bench.dump_outputs(str(tmp_path / "b"), img)
+    a, b = np.load(tmp_path / "a" / "image.npy"), np.load(tmp_path / "b" / "image.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_PIXELS, 4) and a.nbytes <= 64 << 20
+    assert a.tobytes() == b.tobytes()
+    rows = a[:, 0].astype(np.int64) // 4
+    assert (np.diff(rows) > 0).all() and rows[0] >= 0 and rows[-1] < n
+    np.testing.assert_array_equal(a, img[rows])
+    bench.dump_outputs(str(tmp_path / "c"), img[:1000])
+    assert np.load(tmp_path / "c" / "image.npy").tobytes() == img[:1000].tobytes()
