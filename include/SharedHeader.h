@@ -199,9 +199,31 @@ typedef struct ptb_counters {
     uint64_t reserved[3];
 } ptb_counters;
 
+/* ---- scene queries on caller-owned device ray buffers (ptb_scene_intersect) -------------------
+ * One ray = 32 bytes, read with one 256-bit load (the array must be 32-byte aligned).  A query accepts a triangle at
+ * 0 < t < tmax (tmax <= 0 or NaN: a miss); there is no tmin, so callers offset their origins (the reference uses
+ * p + 0.01 * wi).  One hit = 16 bytes: tri = index into the caller's triangle array or -1 (then t = u = v = 0); the
+ * quad id of a hit is tris[tri].id.                                                                             */
+typedef struct ptb_ray {
+    float o[3];
+    float tmax;
+    float d[3];
+    int32_t reserved;
+} ptb_ray;
+typedef struct ptb_hit {
+    float t, u, v;
+    int32_t tri;
+} ptb_hit;
+enum {
+    PTB_QUERY_CLOSEST = 0, /* smallest t; equal t -> lowest caller index                  */
+    PTB_QUERY_ANY = 1      /* the first triangle accepted in traversal order (shadow rays) */
+};
+
 #ifdef __cplusplus
 } /* extern "C" */
 #if __cplusplus >= 201103L
+static_assert(sizeof(ptb_ray) == 32, "ray record must be 32 bytes (one 256-bit load)");
+static_assert(sizeof(ptb_hit) == 16, "hit record must be 16 bytes (one 128-bit store)");
 static_assert(sizeof(ptb_material) == 64, "Material must be 64 bytes (RaytraceTest.cpp:50-59)");
 static_assert(sizeof(ptb_triangle) == 64, "Triangle must be 64 bytes (RaytraceTest.cpp:61-76)");
 static_assert(sizeof(ptb_bvh_node) == 64, "binary BVH node must be 64 bytes");

@@ -193,6 +193,16 @@ int ptb_render_local_pixels(const ptb_render_params* p);
 int ptb_render(ptb_device* dev, ptb_scene* scene, const ptb_render_params* params, ptb_buffer* frame,
                ptb_buffer* stats, ptb_counters* counters);
 
+/* Scene queries on rays that already live on the device (a caller's camera, shadow or visibility rays, a torch pipeline).
+ * rays: n_rays ptb_ray records (>= 32 * n_rays bytes, 32-byte aligned); hits: n_rays ptb_hit records (>= 16 * n_rays bytes);
+ * stats: NULL or 2 x uint32 per ray (BVH nodes fetched, triangle tests started; >= 8 * n_rays bytes).  query = PTB_QUERY_*.
+ * Results, visit and test counts are those of the render paths' queries on the scene's form (FLAT, 4-wide or quantised binary;
+ * DESIGN.md section 4).  Like ptb_render: asynchronous on the device's stream, no allocation per call; counters (host pointer
+ * or NULL) synchronise and return rays_closest / rays_any, and nodes / tri_tests when stats is given; the cumulative mode of
+ * ptb_device_counters applies.  n_rays = 0 does nothing.                                                                 */
+int ptb_scene_intersect(ptb_device* dev, ptb_scene* scene, int query, ptb_buffer* rays, int n_rays, ptb_buffer* hits,
+                        ptb_buffer* stats, ptb_counters* counters);
+
 /* End-to-end convenience with HOST buffers: uploads the scene records (H2D),
  * (re)builds the resident scene if the records changed, renders, reads the frame
  * (and stats) back (D2H) and synchronises.  out_rgba: float4 per local pixel. */

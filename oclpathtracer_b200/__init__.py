@@ -48,6 +48,11 @@ STATS_DTYPE = np.dtype(
         ("visits_secondary", "<u4"), ("count", "<u4"), ("id_hash", "<u4"), ("tri_tests", "<u4"),
     ]
 )
+RAY_DTYPE = np.dtype(  # ptb_ray, 32 bytes (one 256-bit load); arrays must be 32-byte aligned
+    [("o", "<f4", 3), ("tmax", "<f4"), ("d", "<f4", 3), ("reserved", "<i4")]
+)
+HIT_DTYPE = np.dtype([("t", "<f4"), ("u", "<f4"), ("v", "<f4"), ("tri", "<i4")])  # ptb_hit, 16 bytes; tri = -1: miss
+QUERY_CLOSEST, QUERY_ANY = 0, 1
 
 
 class RenderParams(C.Structure):
@@ -99,7 +104,7 @@ EXPORTS = [
     "ptb_bvh_build_host", "ptb_scene_create", "ptb_scene_create_gpu", "ptb_scene_destroy", "ptb_scene_info", "ptb_scene_bvh_width", "ptb_scene_mode_width", "ptb_scene_copy_bvh", "ptb_scene_copy_bvh_quantized",
     "ptb_render_params_default", "ptb_render_local_pixels", "ptb_render", "ptb_render_host",
     "ptb_buffer_ipc_export", "ptb_buffer_ipc_import", "ptb_render_gather",
-    "ptb_render_host_async", "ptb_job_wait", "ptb_host_alloc", "ptb_host_free", "ptb_trace",
+    "ptb_render_host_async", "ptb_job_wait", "ptb_host_alloc", "ptb_host_free", "ptb_trace", "ptb_scene_intersect",
     "ptb_device_add_helper", "ptb_device_helper_count", "ptb_render_multi", "ptb_device_profile", "ptb_device_counters", "ptb_buffer_to_rgb8", "ptb_device_profile_read", "ptb_device_set_tuning", "ptb_test_sincos", "ptb_test_pow", "ptb_test_ieee", "ptb_test_rng", "ptb_test_camera",
 ]
 
@@ -165,6 +170,8 @@ def lib():
         L.ptb_launch_serialize.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int]
         L.ptb_launch_deserialize.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int] + [C.c_void_p] * 5
         L.ptb_trace.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 9
+        L.ptb_scene_intersect.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                          C.c_void_p]
         L.ptb_device_profile.argtypes = [C.c_void_p, C.c_int]
         L.ptb_device_profile_read.argtypes = [C.c_void_p] * 5
         L.ptb_device_set_tuning.argtypes = [C.c_void_p, C.c_int, C.c_int]
@@ -474,6 +481,58 @@ class Device:
                                _p(out["tri"]), _p(out["t"]), _p(out["u"]), _p(out["v"]), _p(out["visits"]),
                                _p(out["tests"])))
         return out
+
+    def intersect(self, scene, rays, hits=None, any_hit=False, stats=None, want_counters=False):
+        """ptb_scene_intersect: closest- (or any-) hit queries on rays that live on this device.
+
+        rays, hits and stats are each a Buffer or a CUDA torch tensor: rays = RAY_DTYPE records (a float32 tensor of shape
+        (n, 8): o.xyz, tmax, d.xyz, unused), hits = HIT_DTYPE records (a float32 (n, 4) tensor: t, u, v and the triangle
+        index as the bits of an int32, read it with `.view(torch.int32)`), stats = NULL or 2 x uint32 per ray (nodes fetched,
+        triangle tests; an int32 (n, 2) tensor).  hits=None allocates them (a tensor for tensor rays, else a Buffer).
+        Tensors are wrapped for the duration of the call; the Device must have been created on torch's current stream, so
+        that the query runs after the work that produced the rays.  Asynchronous unless want_counters.
+        Returns hits, or (hits, counters) when want_counters."""
+        tensors = [x for x in (rays, hits, stats) if x is not None and not isinstance(x, Buffer)]
+        if tensors:
+            import torch
+
+            cur = torch.cuda.current_stream(tensors[0].device).cuda_stream
+            if cur != (self.stream() or 0):  # the legacy default stream is handle 0 (ctypes returns None for it)
+                raise PtbError("Device.intersect: tensors need a Device created on torch.cuda.current_stream() "
+                               "(Device(index, stream=torch.cuda.current_stream().cuda_stream)); "
+                               "on another stream the query would race with the work that wrote the rays")
+            for x in tensors:
+                if not x.is_cuda or not x.is_contiguous() or x.element_size() != 4:
+                    raise PtbError("Device.intersect: tensors must be contiguous CUDA tensors of 4-byte elements")
+        if isinstance(rays, Buffer):
+            n = rays.nbytes // RAY_DTYPE.itemsize
+        else:
+            if rays.dim() != 2 or rays.shape[1] != 8 or rays.dtype != torch.float32:
+                raise PtbError(f"Device.intersect: a ray tensor is float32 of shape (n, 8), got {tuple(rays.shape)} {rays.dtype}")
+            n = rays.shape[0]
+        if hits is None:
+            hits = self.buffer(max(1, n) * HIT_DTYPE.itemsize) if isinstance(rays, Buffer) else \
+                torch.empty((n, 4), dtype=torch.float32, device=rays.device)
+        ctr = Counters() if want_counters else None
+        wrapped = []
+
+        def handle(x):
+            if x is None:
+                return None
+            if isinstance(x, Buffer):
+                return x._h
+            b = Buffer(self, x.numel() * x.element_size(), device_ptr=x.data_ptr())
+            wrapped.append(b)
+            return b._h
+
+        try:
+            if not (n == 0 and tensors):  # an empty tensor has no storage to wrap; the call would be a no-op anyway
+                _check(lib().ptb_scene_intersect(self._h, scene._h, QUERY_ANY if any_hit else QUERY_CLOSEST, handle(rays), n,
+                                                 handle(hits), handle(stats), C.byref(ctr) if ctr is not None else None))
+        finally:
+            for b in wrapped:
+                b.close()
+        return (hits, ctr.as_dict()) if want_counters else hits
 
     def test_sincos(self, x):
         x = np.ascontiguousarray(x, np.float32)

@@ -52,6 +52,7 @@ struct ptb_device {
     void* samples = nullptr; size_t samples_bytes = 0;
     void* sum = nullptr; size_t sum_bytes = 0;
     void* wf = nullptr; size_t wf_bytes = 0;  // wavefront queues
+    void* isect = nullptr; size_t isect_bytes = 0;  // ptb_scene_intersect: work counter of the persistent grid
     unsigned long long* counters = nullptr;   // CTR_COUNT + wavefront queue counters
     std::map<std::string, ptb_kernel*> kernels;  // KernelManager::m_map analogue (Adl/AdlKernel.cpp:142)
     // ptb_render_host cache
@@ -269,6 +270,7 @@ extern "C" int ptb_device_destroy(ptb_device* dev) {
     if (dev->samples) cudaFree(dev->samples);
     if (dev->sum) cudaFree(dev->sum);
     if (dev->wf) cudaFree(dev->wf);
+    if (dev->isect) cudaFree(dev->isect);
     if (dev->counters) cudaFree(dev->counters);
     if (dev->pinned) cudaFreeHost(dev->pinned);
     for (cudaEvent_t e : dev->ev_pool) cudaEventDestroy(e);
@@ -1013,6 +1015,82 @@ extern "C" int ptb_render(ptb_device* dev, ptb_scene* scene, const ptb_render_pa
     if (!frame) return fail(PTB_E_INVALID, "ptb_render: null frame buffer");
     return render_impl(dev, scene, params, static_cast<float4*>(frame->d_ptr), frame->bytes,
                        stats ? static_cast<ptb_pixel_stats*>(stats->d_ptr) : nullptr, stats ? stats->bytes : 0, counters);
+}
+
+// ---- scene queries on caller-owned device ray buffers -------------------------------------------------------------
+// k_intersect: tree forms run a persistent grid (resident CTAs, rays fetched from a work counter in device scratch); FLAT scenes
+// one thread per ray.
+
+template <bool ANY, int SMALL, bool STATS>
+static int launch_intersect_t(ptb_device* dev, const ptd::SceneDev& sc, const float4* rays, float4* hits, uint2* stats, int n) {
+    const int block = 128;
+    const size_t smem = ptd::scene_smem_bytes(sc, true, SMALL, block);
+    auto k = ptd::k_intersect<ANY, SMALL, STATS>;
+    int per_sm = 0;
+    if (int rc = set_smem(k, smem, block, &per_sm)) return rc;
+    long long grid = ((long long)n + block - 1) / block;
+    unsigned int* work = static_cast<unsigned int*>(dev->isect);
+    if (SMALL != ptd::PTD_FLAT) {
+        const long long resident = (long long)per_sm * dev->prop.multiProcessorCount;
+        if (grid > resident) grid = resident;
+        CU_TRY(cudaMemsetAsync(work, 0, sizeof(unsigned int), dev->stream));
+    }
+    k<<<(unsigned)grid, block, smem, dev->stream>>>(sc, rays, hits, stats, (unsigned int)n, work, dev->counters);
+    CU_TRY(cudaGetLastError());
+    dev->kernel_launches += 1;
+    return PTB_OK;
+}
+
+extern "C" int ptb_scene_intersect(ptb_device* dev, ptb_scene* scene, int query, ptb_buffer* rays, int n_rays, ptb_buffer* hits,
+                                   ptb_buffer* stats, ptb_counters* counters) {
+    if (!dev || !scene || !rays || !hits) return fail(PTB_E_INVALID, "ptb_scene_intersect: null device, scene, rays or hits");
+    if (n_rays < 0) return fail(PTB_E_INVALID, "ptb_scene_intersect: n_rays %d < 0", n_rays);
+    if (query != PTB_QUERY_CLOSEST && query != PTB_QUERY_ANY) return fail(PTB_E_INVALID, "ptb_scene_intersect: unknown query %d", query);
+    if (scene->dev != dev) return fail(PTB_E_INVALID, "ptb_scene_intersect: scene belongs to another device");
+    if (rays->dev != dev || hits->dev != dev || (stats && stats->dev != dev))
+        return fail(PTB_E_INVALID, "ptb_scene_intersect: buffer belongs to another device");
+    const size_t n = size_t(n_rays);
+    if (rays->bytes < n * sizeof(ptb_ray)) return fail(PTB_E_INVALID, "ptb_scene_intersect: rays buffer too small (%zu < %zu)", rays->bytes, n * sizeof(ptb_ray));
+    if (hits->bytes < n * sizeof(ptb_hit)) return fail(PTB_E_INVALID, "ptb_scene_intersect: hits buffer too small (%zu < %zu)", hits->bytes, n * sizeof(ptb_hit));
+    if (stats && stats->bytes < n * 8) return fail(PTB_E_INVALID, "ptb_scene_intersect: stats buffer too small (%zu < %zu)", stats->bytes, n * 8);
+    if ((reinterpret_cast<uintptr_t>(rays->d_ptr) & 31u) != 0)
+        return fail(PTB_E_INVALID, "ptb_scene_intersect: rays must be 32-byte aligned (one 256-bit load per ray)");
+    if ((reinterpret_cast<uintptr_t>(hits->d_ptr) & 15u) != 0 || (stats && (reinterpret_cast<uintptr_t>(stats->d_ptr) & 7u) != 0))
+        return fail(PTB_E_INVALID, "ptb_scene_intersect: hits must be 16-byte and stats 8-byte aligned");
+    if (n_rays == 0) {
+        if (counters) std::memset(counters, 0, sizeof *counters);
+        return PTB_OK;
+    }
+    if (set_device(dev)) return PTB_E_CUDA;
+    if (!dev->cumulative_counters) CU_TRY(cudaMemsetAsync(dev->counters, 0, sizeof(unsigned long long) * ptd::CTR_COUNT, dev->stream));
+    {
+        if (int rc = ensure(&dev->isect, &dev->isect_bytes, 256)) return rc;
+        const ptd::SceneDev sc = scene_dev(scene, scene->cls);
+        const float4* r = static_cast<const float4*>(rays->d_ptr);
+        float4* h = static_cast<float4*>(hits->d_ptr);
+        uint2* s = stats ? static_cast<uint2*>(stats->d_ptr) : nullptr;
+        const bool any = query == PTB_QUERY_ANY, st = s != nullptr;
+        const int cls = scene->cls;
+        int rc = fail(PTB_E_INVALID, "ptb_scene_intersect: unreachable");
+#define PTB_ISECT_CASE(A, S, T) if (any == A && cls == S && st == T) rc = launch_intersect_t<A, S, T>(dev, sc, r, h, s, n_rays)
+        PTB_ISECT_CASE(false, ptd::PTD_FLAT, false); PTB_ISECT_CASE(false, ptd::PTD_FLAT, true);
+        PTB_ISECT_CASE(true, ptd::PTD_FLAT, false); PTB_ISECT_CASE(true, ptd::PTD_FLAT, true);
+        PTB_ISECT_CASE(false, ptd::PTD_SMALL4, false); PTB_ISECT_CASE(false, ptd::PTD_SMALL4, true);
+        PTB_ISECT_CASE(true, ptd::PTD_SMALL4, false); PTB_ISECT_CASE(true, ptd::PTD_SMALL4, true);
+        PTB_ISECT_CASE(false, ptd::PTD_LARGE, false); PTB_ISECT_CASE(false, ptd::PTD_LARGE, true);
+        PTB_ISECT_CASE(true, ptd::PTD_LARGE, false); PTB_ISECT_CASE(true, ptd::PTD_LARGE, true);
+#undef PTB_ISECT_CASE
+        if (rc) return rc;
+    }
+    if (counters) {
+        unsigned long long hc[ptd::CTR_COUNT];
+        CU_TRY(cudaMemcpyAsync(hc, dev->counters, sizeof hc, cudaMemcpyDeviceToHost, dev->stream));
+        CU_TRY(cudaStreamSynchronize(dev->stream));
+        std::memset(counters, 0, sizeof *counters);
+        counters->rays_closest = hc[ptd::CTR_CLOSEST]; counters->rays_any = hc[ptd::CTR_ANY];
+        counters->nodes = hc[ptd::CTR_NODES]; counters->tri_tests = hc[ptd::CTR_TESTS];
+    }
+    return PTB_OK;
 }
 
 // ---- image-sharded render that delivers straight into the full images of this rank and its peers ----------------

@@ -413,6 +413,61 @@ __global__ void __launch_bounds__(128) wf_shadow_p(const SceneDev sc, const Rend
     }
 }
 
+// ---- scene queries on caller-owned ray buffers (ptb_scene_intersect) ------------------------------------
+// One ptb_ray = (o.xyz, tmax)(d.xyz, -) read with ONE 256-bit load; one ptb_hit = (t, u, v, caller index | -1) written with ONE
+// 128-bit store (t = u = v = 0 on a miss, as ptb_trace and the oracle report it); stats: (nodes fetched, triangle tests) per ray.
+template <bool STATS>
+struct RayBufIO {
+    const float4* rays;  // 2 x float4 per ray
+    float4* hits;
+    uint2* stats;
+    PTD_FI bool load(unsigned int i, V3& o, V3& d, float& tmax) {
+        float4 a, b;
+        ldg256(rays + 2 * (size_t)i, a, b);
+        o = xyz(a); tmax = a.w; d = xyz(b);
+        return true;
+    }
+    PTD_FI void store(unsigned int i, bool hit, const Hit& h, const QueryStats& qs) {
+        hits[i] = hit ? make_float4(h.t, h.u, h.v, __int_as_float(h.idx)) : make_float4(0.0f, 0.0f, 0.0f, __int_as_float(-1));
+        if constexpr (STATS) stats[i] = make_uint2(qs.visits, qs.tests);
+    }
+};
+
+// Tree forms: the persistent while-while traversal of the wavefront stages (dynamic ray fetch, refill at 8 idle lanes); on the
+// 2M-triangle scene it beat the state-machine form and one thread per ray on camera and any-hit rays and was within 1 % on
+// incoherent closest-hit rays (DESIGN.md section 5).
+// FLAT scenes have no node loop to keep busy: one thread per ray over flat_query, as the wavefront does for them.
+template <bool ANY, int SMALL, bool STATS>
+__global__ void __launch_bounds__(128) k_intersect(const SceneDev sc, const float4* rays, float4* hits, uint2* stats,
+                                                   const unsigned int n_rays, unsigned int* work, unsigned long long* counters) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    Ctx c = stage_scene<true, SMALL>(sc, smem);
+    RayBufIO<STATS> io{rays, hits, stats};
+    uint32_t nrays = 0;
+    QueryStats total{0u, 0u};
+    if constexpr (SMALL == PTD_FLAT) {
+        const unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
+        if (i < n_rays) {
+            V3 o, d;
+            float tmax;
+            io.load(i, o, d, tmax);
+            Hit h;
+            const bool hit = flat_query<ANY, STATS>(c, o, d, tmax, h, total);
+            io.store(i, hit, h, total);
+            nrays = 1;
+        }
+    } else {
+        uint2 lstack_mem[PTD_LSTACK_ENTRIES];
+        if (!SMALL && sc.lstack) c.lstack = lstack_mem;
+        trace_persistent<ANY, SMALL, STATS>(c, io, n_rays, work, 8, nrays, total);
+    }
+    flush_counter(counters, ANY ? CTR_ANY : CTR_CLOSEST, nrays);
+    if (STATS) {
+        flush_counter(counters, CTR_NODES, total.visits);
+        flush_counter(counters, CTR_TESTS, total.tests);
+    }
+}
+
 // ---- shade: full path (GenerateColors.cl:233-257) ---------------------------------------------------
 template <bool BVH, int SMALL, bool STATS>
 __global__ void __launch_bounds__(128) wf_shade_path(const SceneDev sc, const RenderArgs a, const WfBuffers w,
