@@ -742,10 +742,9 @@ static int launch_mega_t(ptb_device* dev, const ptd::SceneDev& sc, const ptd::Re
                     if (a.tune[14] == 2) k = ptd::k_path_sm<SMALL, STATS, 8, 2>;
                     if (a.tune[14] == 4) k = ptd::k_path_sm<SMALL, STATS, 8, 4>;
                 }
-                // Large scenes on the local-memory stack: the form with the path state parked in shared memory (k_path_sm2), 11 CTAs per SM
-                // (40 registers; 9 / 10 / 11 CTAs: 4.86 / 4.90 / 4.93 Grays/s on C5) without statistics.  tune[12] = 1: the registers-only k_path_sm;
-                // 28 / 29 / 30: 8 / 9 / 10 CTAs; 32 / 33: 4 / 8
-                // visits per vote (A/B runs).
+                // Large scenes on the local-memory stack: the form with the path state and the box-test constants parked in shared memory
+                // (k_path_sm2) without statistics: 40 registers and no spills, 12 CTAs per SM.  tune[12] = 1: the registers-only k_path_sm;
+                // 28 / 29 / 30: launch bounds of 8 / 9 / 10 CTAs (46 / 46 / 44 registers, 11 resident CTAs; A/B runs).
                 if constexpr (SMALL == ptd::PTD_LARGE) {
                     if (a.tune[12] != 1 && a.tune[12] != 9 && a.tune[14] == 0 && sc2.lstack && sc2.smem_nodes == 0 && total < (1ll << 31) && a.tune[9] <= 0 && block == 128) {
                         auto k2 = ptd::k_path_sm2<STATS, STATS ? 0 : 11, 6>;
@@ -753,8 +752,6 @@ static int launch_mega_t(ptb_device* dev, const ptd::SceneDev& sc, const ptd::Re
                             if (a.tune[12] == 28) k2 = ptd::k_path_sm2<false, 8, 6>;
                             if (a.tune[12] == 29) k2 = ptd::k_path_sm2<false, 9, 6>;
                             if (a.tune[12] == 30) k2 = ptd::k_path_sm2<false, 10, 6>;
-                            if (a.tune[12] == 32) k2 = ptd::k_path_sm2<false, 10, 4>;
-                            if (a.tune[12] == 33) k2 = ptd::k_path_sm2<false, 10, 8>;
                         }
                         ptd::RenderArgs a2 = a;  // the kernel reads its quorums as plain parameters
                         if (a2.tune[0] <= 0) a2.tune[0] = 4;

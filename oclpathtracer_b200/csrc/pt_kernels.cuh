@@ -162,12 +162,33 @@ struct RayCount {
     uint32_t closest, any;
 };
 
+// The path state that the shading step reads and writes: the ray, the RNG state, the radiance and the throughput mask.
+// PathRegs keeps it in registers; k_path_sm2 keeps it in shared memory (PathCol) and loads each field where it is used.
+struct PathRegs {
+    Ray& r;
+    uint32_t& seed;
+    V3& radiance;
+    V3& mask;
+    V3 hp;  // the hit point
+    PTD_FI V3 o() const { return r.o; }
+    PTD_FI V3 d() const { return r.d; }
+    PTD_FI uint32_t rng() const { return seed; }
+    PTD_FI V3 rad() const { return radiance; }
+    PTD_FI V3 msk() const { return mask; }
+    PTD_FI V3 hit_point() const { return hp; }
+    PTD_FI void set_rng(uint32_t v) { seed = v; }
+    PTD_FI void set_rad(V3 v) { radiance = v; }
+    PTD_FI void set_msk(V3 v) { mask = v; }
+    PTD_FI void set_hit_point(V3 v) { hp = v; }
+    PTD_FI void set_ray(const Ray& v) { r = v; }
+};
+
 // The part of one path-loop iteration that follows the scene query, GenerateColors.cl:233-257: `hit`/`h` are the query's
-// result, `visits` its node visits.  Returns true when the path goes on (r, mask, seed updated), false when it ended;
+// result, `visits` its node visits.  Returns true when the path goes on (ray, mask, seed updated), false when it ended;
 // radiance accumulates either way.
-template <int SMALL, bool STATS>
-PTD_FI bool path_after_hit(const Ctx& c, bool hit, const Hit& h, Ray& r, uint32_t& seed, V3& radiance, V3& mask, int i,
-                           int max_depth, SampleStats<STATS>& st, uint32_t visits) {
+template <int SMALL, bool STATS, class PS>
+PTD_FI bool path_after_hit(const Ctx& c, bool hit, const Hit& h, PS& ps, int i, int max_depth, SampleStats<STATS>& st,
+                           uint32_t visits) {
     V3 p1, e1, e2; int idx = -1, quad = -1;
     if (hit) load_tri<SMALL>(c, h.pos, p1, e1, e2, idx, quad);
     if constexpr (STATS) {
@@ -176,26 +197,41 @@ PTD_FI bool path_after_hit(const Ctx& c, bool hit, const Hit& h, Ray& r, uint32_
         st.count++;
     }
     if (!hit) {  // :233-237, max(bg, 0) = bg
-        radiance = mk(radiance.x + mask.x * 0.45f, radiance.y + mask.y * 0.45f, radiance.z + mask.z * 0.45f);
+        const V3 radiance = ps.rad(), mask = ps.msk();
+        ps.set_rad(mk(radiance.x + mask.x * 0.45f, radiance.y + mask.y * 0.45f, radiance.z + mask.z * 0.45f));
         return false;
     }
     V3 p, n;
-    hit_point_normal(e1, e2, r.o, r.d, h, p, n);
+    hit_point_normal(e1, e2, ps.o(), ps.d(), h, p, n);
+    ps.set_hit_point(p);
     V3 albedo, emissive; float roughness; int type;
     load_mat<SMALL>(c, quad, albedo, roughness, emissive, type);  // :239
-    radiance = mk(radiance.x + mask.x * emissive.x * 3.0f, radiance.y + mask.y * emissive.y * 3.0f,
-                  radiance.z + mask.z * emissive.z * 3.0f);      // :241
+    {
+        const V3 radiance = ps.rad(), mask = ps.msk();
+        ps.set_rad(mk(radiance.x + mask.x * emissive.x * 3.0f, radiance.y + mask.y * emissive.y * 3.0f,
+                      radiance.z + mask.z * emissive.z * 3.0f));  // :241
+    }
     if (i + 1 >= max_depth) return false;  // the last segment's BSDF sample cannot reach the radiance
-    n = dot(n, r.d) < 0.0f ? n : mul(n, -1.0f);                   // :243
+    const V3 d = ps.d();
+    n = dot(n, d) < 0.0f ? n : mul(n, -1.0f);                     // :243
     V3 wi = mk(0.0f, 0.0f, 0.0f);
-    const V3 wo = neg(r.d);                                       // :246
+    const V3 wo = neg(d);                                         // :246
     float pdf = 0.0f;                                             // :247
+    uint32_t seed = ps.rng();
     const V3 color = brdf(wo, wi, pdf, n, albedo, roughness, type, seed);  // :249
+    ps.set_rng(seed);
     if (pdf <= 0.0f) return false;                                // :251
     const float dw = dot(wi, n);
-    mask = mk(mask.x * (color.x * dw / pdf), mask.y * (color.y * dw / pdf), mask.z * (color.z * dw / pdf));  // :253-255
-    r = get_ray(add(p, mul(wi, 0.01f)), wi);                      // :257
+    const V3 mask = ps.msk();
+    ps.set_msk(mk(mask.x * (color.x * dw / pdf), mask.y * (color.y * dw / pdf), mask.z * (color.z * dw / pdf)));  // :253-255
+    ps.set_ray(get_ray(add(ps.hit_point(), mul(wi, 0.01f)), wi));  // :257
     return true;
+}
+template <int SMALL, bool STATS>
+PTD_FI bool path_after_hit(const Ctx& c, bool hit, const Hit& h, Ray& r, uint32_t& seed, V3& radiance, V3& mask, int i,
+                           int max_depth, SampleStats<STATS>& st, uint32_t visits) {
+    PathRegs ps{r, seed, radiance, mask, {}};
+    return path_after_hit<SMALL, STATS>(c, hit, h, ps, i, max_depth, st, visits);
 }
 
 // One iteration of the path loop, GenerateColors.cl:229-258: the scene query, then path_after_hit.
@@ -684,8 +720,38 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm(const SceneDev sc, const 
 // local-memory stack and no staged prefix only; per-sample arithmetic and order unchanged.  Measured on C5 (same kernel body,
 // 6 visits per vote): registers only, 8 CTAs 4.36 Grays/s; parked, 8 / 9 / 10 / 11 CTAs (64 / 56 / 48 / 40 registers): 4.43 / 4.58 /
 // 4.61 / 4.62 with the old quorums, 4.69 at 10 CTAs with the re-tuned ones.
-enum { PK_OX = 0, PK_OY, PK_OZ, PK_DX, PK_DY, PK_DZ, PK_U, PK_V, PK_POS, PK_IDX, PK_RX, PK_RY, PK_RZ, PK_MX, PK_MY, PK_MZ, PK_SEED, PK_SLOT, PK_DEPTH, PK_FIELDS };
+// A node visit or a shade step runs only for the lanes in that state, but registers belong to threads: whatever one lane keeps in
+// registers across a phase, every lane pays for.  So the box-test constants (RayPre, 9 words) live in the column too: written once
+// per query by begin_query and loaded by the node phase at each vote; and the shading step (path_after_hit over PathCol) loads each
+// field where it uses it and stores it back as soon as it is final.  At the 40-register cap of 12 CTAs per SM nothing spills
+// (it spilled 128 B per thread when RayPre and the loaded path state were held across the shade phase).
+enum { PK_OX = 0, PK_OY, PK_OZ, PK_DX, PK_DY, PK_DZ, PK_U, PK_V, PK_POS, PK_IDX, PK_RX, PK_RY, PK_RZ, PK_MX, PK_MY, PK_MZ, PK_SEED, PK_SLOT, PK_DEPTH,
+       PK_AX, PK_AY, PK_AZ, PK_BX, PK_BY, PK_BZ, PK_SN0, PK_SN1, PK_SN2, PK_FIELDS };
 static inline size_t path_sm2_smem_bytes(int block) { return 16 + (size_t)PK_FIELDS * block * 4; }
+constexpr uint32_t PK_STRIDE = 128u * 4u;  // the launcher runs k_path_sm2 with 128-thread CTAs only: field offsets are immediates
+
+// path_after_hit's path state in a lane's shared-memory column (pk: the address of its word 0).  Each field is loaded where the
+// shading step uses it and stored as soon as it is final, so that no field stays in a register across the step.
+struct PathCol {
+    uint32_t pk;
+    Ray r;  // the last ray set_ray stored, for the query that follows
+    PTD_FI float ldf(int f) const { return __uint_as_float(lds32(pk + (uint32_t)f * PK_STRIDE)); }
+    PTD_FI void stf(int f, float v) const { sts32(pk + (uint32_t)f * PK_STRIDE, __float_as_uint(v)); }
+    PTD_FI V3 o() const { return mk(ldf(PK_OX), ldf(PK_OY), ldf(PK_OZ)); }
+    PTD_FI V3 d() const { return mk(ldf(PK_DX), ldf(PK_DY), ldf(PK_DZ)); }
+    PTD_FI uint32_t rng() const { return lds32(pk + PK_SEED * PK_STRIDE); }
+    PTD_FI V3 rad() const { return mk(ldf(PK_RX), ldf(PK_RY), ldf(PK_RZ)); }
+    PTD_FI V3 msk() const { return mk(ldf(PK_MX), ldf(PK_MY), ldf(PK_MZ)); }
+    PTD_FI V3 hit_point() const { return o(); }  // the hit point replaces the origin, which is dead once it is known
+    PTD_FI void set_rng(uint32_t v) { sts32(pk + PK_SEED * PK_STRIDE, v); }
+    PTD_FI void set_rad(V3 v) { stf(PK_RX, v.x); stf(PK_RY, v.y); stf(PK_RZ, v.z); }
+    PTD_FI void set_msk(V3 v) { stf(PK_MX, v.x); stf(PK_MY, v.y); stf(PK_MZ, v.z); }
+    PTD_FI void set_hit_point(V3 v) { stf(PK_OX, v.x); stf(PK_OY, v.y); stf(PK_OZ, v.z); }
+    PTD_FI void set_ray(const Ray& v) {
+        r = v;
+        stf(PK_OX, v.o.x); stf(PK_OY, v.o.y); stf(PK_OZ, v.o.z); stf(PK_DX, v.d.x); stf(PK_DY, v.d.y); stf(PK_DZ, v.d.z);
+    }
+};
 
 template <bool STATS, int MINB, int NSTEP>
 __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const RenderArgs a, unsigned long long* work_counter) {
@@ -695,11 +761,10 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
     c.lstack = lstack_mem + 1;
     uint32_t pk = smem_u32(smem) + 16u + threadIdx.x * 4u;
     asm volatile("" : "+r"(pk));  // opaque: kept in a register instead of being re-derived (S2R + shared-window base + LEA, 7 instructions) at every vote
-    constexpr uint32_t fstride = 128u * 4u;  // the launcher runs this kernel with 128-thread CTAs only: field offsets are immediates
-#define PKL(f) lds32(pk + (uint32_t)(f) * fstride)
-#define PKLF(f) __uint_as_float(lds32(pk + (uint32_t)(f) * fstride))
-#define PKS(f, v) sts32(pk + (uint32_t)(f) * fstride, (uint32_t)(v))
-#define PKSF(f, v) sts32(pk + (uint32_t)(f) * fstride, __float_as_uint(v))
+#define PKL(f) lds32(pk + (uint32_t)(f) * PK_STRIDE)
+#define PKLF(f) __uint_as_float(lds32(pk + (uint32_t)(f) * PK_STRIDE))
+#define PKS(f, v) sts32(pk + (uint32_t)(f) * PK_STRIDE, (uint32_t)(v))
+#define PKSF(f, v) sts32(pk + (uint32_t)(f) * PK_STRIDE, __float_as_uint(v))
     const uint32_t total = (uint32_t)((long long)a.frames_in_batch * a.n_local);  // the launcher guarantees < 2^31 slots
     const unsigned lane = threadIdx.x & 31u;
     // quorums, resolved by the launcher (defaults re-tuned for 10 resident CTAs: shade 16 / 20 / 24 -> 4.61 / 4.66 / 4.51,
@@ -711,7 +776,6 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
     bool exhausted = false;
     int li = 0, frame = 0;  // STATS only
     uint32_t tests0 = 0, visits0 = 0;
-    RayPre rp{mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 0.f), {0u, 0u, 0u}};
     float best_t = 1e20f;
     int cur = 0, sp = 0;
     SampleStats<STATS> st{};
@@ -719,7 +783,9 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
         visits0 = qs.visits;
         best_t = 1e20f;
         PKS(PK_IDX, -1);
-        rp = ray_pre<PTD_LARGE>(c, r.o, r.d);
+        const RayPre q = ray_pre<PTD_LARGE>(c, r.o, r.d);
+        PKSF(PK_AX, q.a.x); PKSF(PK_AY, q.a.y); PKSF(PK_AZ, q.a.z); PKSF(PK_BX, q.b.x); PKSF(PK_BY, q.b.y); PKSF(PK_BZ, q.b.z);
+        PKS(PK_SN0, q.sn[0]); PKS(PK_SN1, q.sn[1]); PKS(PK_SN2, q.sn[2]);
         cur = 0; sp = 0;
         state = ST_NODE;
     };
@@ -752,6 +818,7 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
             }
             if (!n_node || n_shade >= thr_shade) break;
             if (state == ST_NODE) {
+                const RayPre rp{mk(PKLF(PK_AX), PKLF(PK_AY), PKLF(PK_AZ)), mk(PKLF(PK_BX), PKLF(PK_BY), PKLF(PK_BZ)), {PKL(PK_SN0), PKL(PK_SN1), PKL(PK_SN2)}};
                 bool more = node_step2_bf<STATS>(c, rp, best_t, cur, sp, qs);
 #pragma unroll
                 for (int rep = 1; rep < NSTEP; ++rep)
@@ -760,18 +827,16 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
             }
         }
         if (state == ST_SHADE) {
-            Ray r{mk(PKLF(PK_OX), PKLF(PK_OY), PKLF(PK_OZ)), mk(PKLF(PK_DX), PKLF(PK_DY), PKLF(PK_DZ))};
-            V3 radiance = mk(PKLF(PK_RX), PKLF(PK_RY), PKLF(PK_RZ)), mask = mk(PKLF(PK_MX), PKLF(PK_MY), PKLF(PK_MZ));
-            uint32_t seed = PKL(PK_SEED);
-            int depth = (int)PKL(PK_DEPTH);
             Hit h;
             h.idx = (int)PKL(PK_IDX);
             const bool hit = h.idx >= 0;
             h.t = best_t; h.u = PKLF(PK_U); h.v = PKLF(PK_V); h.pos = (int)PKL(PK_POS);
+            const int depth = (int)PKL(PK_DEPTH);
             rc.closest++;
-            const bool more = path_after_hit<PTD_LARGE, STATS>(c, hit, h, r, seed, radiance, mask, depth, a.max_depth, st, qs.visits - visits0);
-            ++depth;
-            if (!more || depth >= a.max_depth) {
+            PathCol ps{pk, {}};
+            const bool more = path_after_hit<PTD_LARGE, STATS>(c, hit, h, ps, depth, a.max_depth, st, qs.visits - visits0);
+            if (!more || depth + 1 >= a.max_depth) {
+                const V3 radiance = ps.rad();
                 a.samples[PKL(PK_SLOT)] = make_float4(cl_max(radiance.x, 0.0f), cl_max(radiance.y, 0.0f), cl_max(radiance.z, 0.0f), 1.0f);  // :260
                 if constexpr (STATS) {
                     if (a.stats && frame == a.stats_frame) {
@@ -782,11 +847,8 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
                 }
                 state = exhausted ? ST_DONE : ST_REGEN;
             } else {
-                PKSF(PK_OX, r.o.x); PKSF(PK_OY, r.o.y); PKSF(PK_OZ, r.o.z); PKSF(PK_DX, r.d.x); PKSF(PK_DY, r.d.y); PKSF(PK_DZ, r.d.z);
-                PKSF(PK_RX, radiance.x); PKSF(PK_RY, radiance.y); PKSF(PK_RZ, radiance.z);
-                PKSF(PK_MX, mask.x); PKSF(PK_MY, mask.y); PKSF(PK_MZ, mask.z);
-                PKS(PK_SEED, seed); PKS(PK_DEPTH, depth);
-                begin_query(r);
+                PKS(PK_DEPTH, depth + 1);
+                begin_query(ps.r);
             }
         }
         const unsigned m_regen = __ballot_sync(0xffffffffu, state == ST_REGEN);
