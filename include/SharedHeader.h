@@ -219,11 +219,24 @@ enum {
     PTB_QUERY_ANY = 1      /* the first triangle accepted in traversal order (shadow rays) */
 };
 
+/* ---- render-mode samples along caller-owned device rays (ptb_scene_shade) -------------------------------------------
+ * One sample = 32 bytes, read with one 256-bit load (the array must be 32-byte aligned).  seed is the RNG state of the sample
+ * (GenerateColors.cl:47-71) after whatever draws the caller's camera made: the reference's camera starts from
+ * gid + hash_uint32(frame) (:308) and draws two floats for its jitter (:278-279).  d need not be normalised; the render
+ * modes use it as given.                                                                                               */
+typedef struct ptb_sample_ray {
+    float o[3];
+    uint32_t seed;
+    float d[3];
+    int32_t reserved; /* ignored */
+} ptb_sample_ray;
+
 #ifdef __cplusplus
 } /* extern "C" */
 #if __cplusplus >= 201103L
 static_assert(sizeof(ptb_ray) == 32, "ray record must be 32 bytes (one 256-bit load)");
 static_assert(sizeof(ptb_hit) == 16, "hit record must be 16 bytes (one 128-bit store)");
+static_assert(sizeof(ptb_sample_ray) == 32, "sample ray record must be 32 bytes (one 256-bit load)");
 static_assert(sizeof(ptb_material) == 64, "Material must be 64 bytes (RaytraceTest.cpp:50-59)");
 static_assert(sizeof(ptb_triangle) == 64, "Triangle must be 64 bytes (RaytraceTest.cpp:61-76)");
 static_assert(sizeof(ptb_bvh_node) == 64, "binary BVH node must be 64 bytes");

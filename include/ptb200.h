@@ -203,6 +203,22 @@ int ptb_render(ptb_device* dev, ptb_scene* scene, const ptb_render_params* param
 int ptb_scene_intersect(ptb_device* dev, ptb_scene* scene, int query, ptb_buffer* rays, int n_rays, ptb_buffer* hits,
                         ptb_buffer* stats, ptb_counters* counters);
 
+/* Render-mode samples along rays that already live on the device (another viewpoint or lens, adaptively chosen pixels, rays a
+ * torch pipeline produced).  Sample i is exactly what ptb_render computes for one pixel-frame after its camera step, with
+ * rays[i].o, rays[i].d and rays[i].seed in place of the camera ray and the post-camera RNG state (ptb_sample_ray).
+ *   rays      n_rays ptb_sample_ray records (>= 32 * n_rays bytes, 32-byte aligned)
+ *   radiance  float4 per ray (>= 16 * n_rays bytes, 16-byte aligned): xyz after max(., 0), w = 1, the value ptb_render writes
+ *             into a sample slot
+ *   stats     NULL or ptb_pixel_stats per ray (>= 32 * n_rays bytes, 16-byte aligned), fields as for ptb_render
+ * Read from params: mode, max_depth, ao_samples, ao_max_dist, light_quad and light_p1 / ea / eb (the light comes from light_quad
+ * when ea is all zero, as for ptb_render).  Ignored: the image size, frames, accum, shard, output and frames_per_batch.
+ * Refused: accel = PTB_ACCEL_BRUTE and integrator = PTB_INTEGRATOR_WAVEFRONT.  Every closest-hit query runs to tmax 1e20, as
+ * the reference's do.  Asynchronous on the device's stream, no allocation per call; counters (host pointer or NULL)
+ * synchronise and return the rays, nodes and tri_tests (with stats) and samples = n_rays; the cumulative mode of
+ * ptb_device_counters applies.  n_rays = 0 does nothing.                                                              */
+int ptb_scene_shade(ptb_device* dev, ptb_scene* scene, const ptb_render_params* params, ptb_buffer* rays, int n_rays,
+                    ptb_buffer* radiance, ptb_buffer* stats, ptb_counters* counters);
+
 /* End-to-end convenience with HOST buffers: uploads the scene records (H2D),
  * (re)builds the resident scene if the records changed, renders, reads the frame
  * (and stats) back (D2H) and synchronises.  out_rgba: float4 per local pixel. */

@@ -52,6 +52,9 @@ RAY_DTYPE = np.dtype(  # ptb_ray, 32 bytes (one 256-bit load); arrays must be 32
     [("o", "<f4", 3), ("tmax", "<f4"), ("d", "<f4", 3), ("reserved", "<i4")]
 )
 HIT_DTYPE = np.dtype([("t", "<f4"), ("u", "<f4"), ("v", "<f4"), ("tri", "<i4")])  # ptb_hit, 16 bytes; tri = -1: miss
+SAMPLE_RAY_DTYPE = np.dtype(  # ptb_sample_ray, 32 bytes (one 256-bit load); seed = the sample's RNG state after the camera's draws
+    [("o", "<f4", 3), ("seed", "<u4"), ("d", "<f4", 3), ("reserved", "<i4")]
+)
 QUERY_CLOSEST, QUERY_ANY = 0, 1
 
 
@@ -104,7 +107,7 @@ EXPORTS = [
     "ptb_bvh_build_host", "ptb_scene_create", "ptb_scene_create_gpu", "ptb_scene_destroy", "ptb_scene_info", "ptb_scene_bvh_width", "ptb_scene_mode_width", "ptb_scene_copy_bvh", "ptb_scene_copy_bvh_quantized",
     "ptb_render_params_default", "ptb_render_local_pixels", "ptb_render", "ptb_render_host",
     "ptb_buffer_ipc_export", "ptb_buffer_ipc_import", "ptb_render_gather",
-    "ptb_render_host_async", "ptb_job_wait", "ptb_host_alloc", "ptb_host_free", "ptb_trace", "ptb_scene_intersect",
+    "ptb_render_host_async", "ptb_job_wait", "ptb_host_alloc", "ptb_host_free", "ptb_trace", "ptb_scene_intersect", "ptb_scene_shade",
     "ptb_device_add_helper", "ptb_device_helper_count", "ptb_render_multi", "ptb_device_profile", "ptb_device_counters", "ptb_buffer_to_rgb8", "ptb_device_profile_read", "ptb_device_set_tuning", "ptb_test_sincos", "ptb_test_pow", "ptb_test_ieee", "ptb_test_rng", "ptb_test_camera",
 ]
 
@@ -172,6 +175,7 @@ def lib():
         L.ptb_trace.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 9
         L.ptb_scene_intersect.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                           C.c_void_p]
+        L.ptb_scene_shade.argtypes = [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 3
         L.ptb_device_profile.argtypes = [C.c_void_p, C.c_int]
         L.ptb_device_profile_read.argtypes = [C.c_void_p] * 5
         L.ptb_device_set_tuning.argtypes = [C.c_void_p, C.c_int, C.c_int]
@@ -492,21 +496,12 @@ class Device:
         Tensors are wrapped for the duration of the call; the Device must have been created on torch's current stream, so
         that the query runs after the work that produced the rays.  Asynchronous unless want_counters.
         Returns hits, or (hits, counters) when want_counters."""
-        tensors = [x for x in (rays, hits, stats) if x is not None and not isinstance(x, Buffer)]
-        if tensors:
-            import torch
-
-            cur = torch.cuda.current_stream(tensors[0].device).cuda_stream
-            if cur != (self.stream() or 0):  # the legacy default stream is handle 0 (ctypes returns None for it)
-                raise PtbError("Device.intersect: tensors need a Device created on torch.cuda.current_stream() "
-                               "(Device(index, stream=torch.cuda.current_stream().cuda_stream)); "
-                               "on another stream the query would race with the work that wrote the rays")
-            for x in tensors:
-                if not x.is_cuda or not x.is_contiguous() or x.element_size() != 4:
-                    raise PtbError("Device.intersect: tensors must be contiguous CUDA tensors of 4-byte elements")
+        args = _CallArgs(self, "Device.intersect", rays, hits, stats)
         if isinstance(rays, Buffer):
             n = rays.nbytes // RAY_DTYPE.itemsize
         else:
+            import torch
+
             if rays.dim() != 2 or rays.shape[1] != 8 or rays.dtype != torch.float32:
                 raise PtbError(f"Device.intersect: a ray tensor is float32 of shape (n, 8), got {tuple(rays.shape)} {rays.dtype}")
             n = rays.shape[0]
@@ -514,25 +509,43 @@ class Device:
             hits = self.buffer(max(1, n) * HIT_DTYPE.itemsize) if isinstance(rays, Buffer) else \
                 torch.empty((n, 4), dtype=torch.float32, device=rays.device)
         ctr = Counters() if want_counters else None
-        wrapped = []
-
-        def handle(x):
-            if x is None:
-                return None
-            if isinstance(x, Buffer):
-                return x._h
-            b = Buffer(self, x.numel() * x.element_size(), device_ptr=x.data_ptr())
-            wrapped.append(b)
-            return b._h
-
-        try:
-            if not (n == 0 and tensors):  # an empty tensor has no storage to wrap; the call would be a no-op anyway
-                _check(lib().ptb_scene_intersect(self._h, scene._h, QUERY_ANY if any_hit else QUERY_CLOSEST, handle(rays), n,
-                                                 handle(hits), handle(stats), C.byref(ctr) if ctr is not None else None))
-        finally:
-            for b in wrapped:
-                b.close()
+        with args:
+            if not (n == 0 and args.tensors):  # an empty tensor has no storage to wrap; the call would be a no-op anyway
+                _check(lib().ptb_scene_intersect(self._h, scene._h, QUERY_ANY if any_hit else QUERY_CLOSEST, args.handle(rays), n,
+                                                 args.handle(hits), args.handle(stats), C.byref(ctr) if ctr is not None else None))
         return (hits, ctr.as_dict()) if want_counters else hits
+
+    def shade(self, scene, params, rays, radiance=None, stats=None, want_counters=False):
+        """ptb_scene_shade: render-mode samples (params.mode, max_depth, ao_samples, ao_max_dist, light) along rays that live on
+        this device; sample i is what render() computes for one pixel-frame after its camera step, with ray i and its seed.
+
+        rays, radiance and stats are each a Buffer or a contiguous CUDA torch tensor: rays = SAMPLE_RAY_DTYPE records (an (n, 8)
+        tensor of any 4-byte dtype: o.xyz, the seed as the bits of a uint32, d.xyz, unused), radiance = float4 per ray (a
+        float32 (n, 4) tensor: xyz, w = 1), stats = NULL or STATS_DTYPE per ray (an int32 (n, 8) tensor).  radiance=None
+        allocates it (a tensor for tensor rays, else a Buffer).  The Device must have been created on torch's current stream
+        when tensors are used.  Asynchronous unless want_counters.  Returns radiance, or (radiance, counters) when
+        want_counters."""
+        args = _CallArgs(self, "Device.shade", rays, radiance, stats)
+        if isinstance(rays, Buffer):
+            n = rays.nbytes // SAMPLE_RAY_DTYPE.itemsize
+        else:
+            import torch
+
+            if rays.dim() != 2 or rays.shape[1] != 8:
+                raise PtbError(f"Device.shade: a ray tensor has shape (n, 8), got {tuple(rays.shape)}")
+            n = rays.shape[0]
+            for x, name, dt, cols in ((radiance, "radiance", torch.float32, 4), (stats, "stats", torch.int32, 8)):
+                if x is not None and not isinstance(x, Buffer) and (x.dtype != dt or x.dim() != 2 or tuple(x.shape) != (n, cols)):
+                    raise PtbError(f"Device.shade: {name} is a {dt} tensor of shape ({n}, {cols}), got {tuple(x.shape)} {x.dtype}")
+        if radiance is None:
+            radiance = self.buffer(max(1, n) * 16) if isinstance(rays, Buffer) else \
+                torch.empty((n, 4), dtype=torch.float32, device=rays.device)
+        ctr = Counters() if want_counters else None
+        with args:
+            if not (n == 0 and args.tensors):  # an empty tensor has no storage to wrap; the call would be a no-op anyway
+                _check(lib().ptb_scene_shade(self._h, scene._h, C.byref(params), args.handle(rays), n, args.handle(radiance),
+                                             args.handle(stats), C.byref(ctr) if ctr is not None else None))
+        return (radiance, ctr.as_dict()) if want_counters else radiance
 
     def test_sincos(self, x):
         x = np.ascontiguousarray(x, np.float32)
@@ -565,6 +578,49 @@ class Device:
         o, d, s = np.empty((n, 3), np.float32), np.empty((n, 3), np.float32), np.empty(n, np.uint32)
         _check(lib().ptb_test_camera(self._h, width, height, frame, n, _p(gids), _p(o), _p(d), _p(s)))
         return o, d, s
+
+
+
+class _CallArgs:
+    """Buffers or CUDA torch tensors as ptb_buffer handles for one call of `what` (Device.intersect, Device.shade).
+
+    Tensors must be contiguous CUDA tensors of 4-byte elements, and the Device must have been created on torch's current
+    stream: on another stream the call would race with the work that wrote its inputs.  Used as a context manager, the
+    wrappers made by handle() are released when the call returns."""
+
+    def __init__(self, dev, what, *xs):
+        self.dev = dev
+        self.tensors = [x for x in xs if x is not None and not isinstance(x, Buffer)]
+        self.wrapped = []
+        if self.tensors:
+            import torch
+
+            cur = torch.cuda.current_stream(self.tensors[0].device).cuda_stream
+            if cur != (dev.stream() or 0):  # the legacy default stream is handle 0 (ctypes returns None for it)
+                raise PtbError(f"{what}: tensors need a Device created on torch.cuda.current_stream() "
+                               "(Device(index, stream=torch.cuda.current_stream().cuda_stream)); "
+                               "on another stream the query would race with the work that wrote the rays")
+            for x in self.tensors:
+                if not x.is_cuda or not x.is_contiguous() or x.element_size() != 4:
+                    raise PtbError(f"{what}: tensors must be contiguous CUDA tensors of 4-byte elements")
+
+    def handle(self, x):
+        if x is None:
+            return None
+        if isinstance(x, Buffer):
+            return x._h
+        b = Buffer(self.dev, x.numel() * x.element_size(), device_ptr=x.data_ptr())
+        self.wrapped.append(b)
+        return b._h
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        for b in self.wrapped:
+            b.close()
+        self.wrapped = []
+        return False
 
 
 class Buffer:

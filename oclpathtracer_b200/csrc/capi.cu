@@ -862,6 +862,30 @@ static int validate(const ptb_render_params* p) {
     return PTB_OK;
 }
 
+// The area light of the render args (ptb_render and ptb_scene_shade): light_p1 / ea / eb from the params, or derived from the
+// triangles of light_quad when ea is all zero (DIRECT only); for DIRECT also |cross(ea, eb)| and its unit vector, the same for
+// every sample.
+static int setup_light(const ptb_scene* scene, const ptb_render_params* p, ptd::RenderArgs& a) {
+    a.light_quad = p->light_quad;
+    const bool have_light = p->light_ea[0] != 0.f || p->light_ea[1] != 0.f || p->light_ea[2] != 0.f;
+    if (have_light) {
+        std::memcpy(a.light_p1, p->light_p1, 12); std::memcpy(a.light_ea, p->light_ea, 12); std::memcpy(a.light_eb, p->light_eb, 12);
+    } else if (p->mode == PTB_MODE_DIRECT) {
+        if (int rc = ptb_light_from_quad(scene->host_tris.data(), scene->n_tris, p->light_quad, a.light_p1, a.light_ea, a.light_eb)) return rc;
+    }
+    if (p->mode == PTB_MODE_DIRECT) {
+        // |cross(ea, eb)| and its unit vector, spelled as the kernels (and the oracle) spell them per sample: products and
+        // sums rounded one by one (this file is compiled without FMA contraction), IEEE sqrt and division
+        const float* ea = a.light_ea; const float* eb = a.light_eb;
+        const float cx = ea[1] * eb[2] - ea[2] * eb[1], cy = ea[2] * eb[0] - ea[0] * eb[2], cz = ea[0] * eb[1] - ea[1] * eb[0];
+        const float dd = (cx * cx + cy * cy) + cz * cz;
+        a.light_area = std::sqrt(dd);
+        const float inv = 1.0f / std::sqrt(dd);
+        a.light_n[0] = cx * inv; a.light_n[1] = cy * inv; a.light_n[2] = cz * inv;
+    }
+    return PTB_OK;
+}
+
 // `ext_samples` + `phase` split one call for the frame-ahead batching of ptb_launch1d: PHASE_TRACE writes the samples of
 // all n_frames into ext_samples and stops; PHASE_RESOLVE folds n_frames already-traced frames from ext_samples into d_frame.
 enum { PHASE_BOTH = 0, PHASE_TRACE = 1, PHASE_RESOLVE = 2 };
@@ -913,25 +937,9 @@ static int render_impl(ptb_device* dev, ptb_scene* scene, const ptb_render_param
     a.width = p->width; a.height = p->height;
     a.n_local = n_local;
     a.max_depth = p->max_depth; a.ao_samples = p->ao_samples; a.ao_max_dist = p->ao_max_dist;
-    a.light_quad = p->light_quad;
-    const bool have_light = p->light_ea[0] != 0.f || p->light_ea[1] != 0.f || p->light_ea[2] != 0.f;
-    if (have_light) {
-        std::memcpy(a.light_p1, p->light_p1, 12); std::memcpy(a.light_ea, p->light_ea, 12); std::memcpy(a.light_eb, p->light_eb, 12);
-    } else if (p->mode == PTB_MODE_DIRECT) {
-        if (int rc = ptb_light_from_quad(scene->host_tris.data(), scene->n_tris, p->light_quad, a.light_p1, a.light_ea, a.light_eb)) return rc;
-    }
+    if (int rc = setup_light(scene, p, a)) return rc;
     a.cam_inv_w = 1.0f / (float)p->width; a.cam_inv_h = 1.0f / (float)p->height;  // GenerateColors.cl:265
     a.cam_aspect = (float)p->width / (float)p->height;                            // :266
-    if (p->mode == PTB_MODE_DIRECT) {
-        // |cross(ea, eb)| and its unit vector, spelled as the kernels (and the oracle) spell them per sample: products and
-        // sums rounded one by one (this file is compiled without FMA contraction), IEEE sqrt and division
-        const float* ea = a.light_ea; const float* eb = a.light_eb;
-        const float cx = ea[1] * eb[2] - ea[2] * eb[1], cy = ea[2] * eb[0] - ea[0] * eb[2], cz = ea[0] * eb[1] - ea[1] * eb[0];
-        const float dd = (cx * cx + cy * cy) + cz * cz;
-        a.light_area = std::sqrt(dd);
-        const float inv = 1.0f / std::sqrt(dd);
-        a.light_n[0] = cx * inv; a.light_n[1] = cy * inv; a.light_n[2] = cz * inv;
-    }
     a.shard.index = p->shard_index; a.shard.count = p->shard_count < 1 ? 1 : p->shard_count; a.shard.block = p->shard_block < 1 ? 1 : p->shard_block;
     a.samples = ext_samples ? ext_samples : static_cast<float4*>(dev->samples);
     // One frame with accum = LINEAR: the mean of one sample is the sample (0 + c = c and c / 1 = c exactly, w = 1), and without image
@@ -1086,6 +1094,130 @@ extern "C" int ptb_scene_intersect(ptb_device* dev, ptb_scene* scene, int query,
         std::memset(counters, 0, sizeof *counters);
         counters->rays_closest = hc[ptd::CTR_CLOSEST]; counters->rays_any = hc[ptd::CTR_ANY];
         counters->nodes = hc[ptd::CTR_NODES]; counters->tri_tests = hc[ptd::CTR_TESTS];
+    }
+    return PTB_OK;
+}
+
+// ---- render-mode samples along caller-owned device rays -----------------------------------------------------------------
+// The kernels ptb_render's megakernel path launches for the mode's scene form, with their default selection, and the ray
+// source ptd::SampleRays in place of the camera: PRIMARY / AO / DIRECT run k_mega (one thread per ray); PATH runs k_path_sm2 on
+// large scenes with the local-memory stack and k_mega_path_regen elsewhere (FLAT scenes with the warp-pooled triangle phase).
+
+template <int MODE, int SMALL, bool STATS>
+static int launch_shade_t(ptb_device* dev, const ptd::SceneDev& sc, const ptd::ShadeArgs& a) {
+    const int block = 128;
+    const long long n = a.n_local;
+    int per_sm = 0;
+    if constexpr (MODE == PTB_MODE_PATH) {
+        const long long need = (n + block - 1) / block;
+        unsigned long long* work = dev->counters + 32;  // the path kernels' work counter
+        CU_TRY(cudaMemsetAsync(work, 0, sizeof(unsigned long long), dev->stream));
+        if (SMALL == ptd::PTD_LARGE && sc.lstack) {
+            ptd::SceneDev sc2 = sc;
+            sc2.smem_nodes = 0;  // k_path_sm2 fetches every node from global memory
+            auto k2 = ptd::k_path_sm2_rays<STATS, STATS ? 0 : 11, 6>;
+            ptd::ShadeArgs a2 = a;  // quorums resolved as for ptb_render
+            if (a2.tune[0] <= 0) a2.tune[0] = 4;
+            if (a2.tune[10] <= 0) a2.tune[10] = 20;
+            if (a2.tune[11] <= 0) a2.tune[11] = 10;
+            const size_t sm2 = ptd::path_sm2_smem_bytes(block);
+            if (int rc = set_smem(k2, sm2, block, &per_sm)) return rc;
+            long long grid = (long long)per_sm * dev->prop.multiProcessorCount;
+            if (grid > need) grid = need;
+            k2<<<(unsigned)grid, block, sm2, dev->stream>>>(sc2, a2, work);
+        } else {
+            auto k = ptd::k_mega_path_regen<true, SMALL, STATS, SMALL == ptd::PTD_FLAT, ptd::SampleRays>;
+            const size_t smem = ptd::scene_smem_bytes(sc, true, SMALL, block);
+            if (int rc = set_smem(k, smem, block, &per_sm)) return rc;
+            long long grid = (long long)per_sm * dev->prop.multiProcessorCount;
+            if (grid > need) grid = need;
+            k<<<(unsigned)grid, block, smem, dev->stream>>>(sc, a, work);
+        }
+    } else {
+        auto k = ptd::k_mega<MODE, true, SMALL, STATS, ptd::SampleRays>;
+        const size_t smem = ptd::scene_smem_bytes(sc, true, SMALL, block);
+        if (int rc = set_smem(k, smem, block)) return rc;
+        k<<<(unsigned)((n + block - 1) / block), block, smem, dev->stream>>>(sc, a);
+    }
+    CU_TRY(cudaGetLastError());
+    dev->kernel_launches += 1;
+    return PTB_OK;
+}
+
+template <int MODE>
+static int launch_shade_m(ptb_device* dev, const ptd::SceneDev& sc, const ptd::ShadeArgs& a, int small, bool stats) {
+#define PTB_SHADE_CASE(S, T) if (small == S && stats == T) return launch_shade_t<MODE, S, T>(dev, sc, a)
+    PTB_SHADE_CASE(ptd::PTD_FLAT, false); PTB_SHADE_CASE(ptd::PTD_FLAT, true);
+    PTB_SHADE_CASE(ptd::PTD_SMALL4, false); PTB_SHADE_CASE(ptd::PTD_SMALL4, true);
+    PTB_SHADE_CASE(ptd::PTD_LARGE, false); PTB_SHADE_CASE(ptd::PTD_LARGE, true);
+#undef PTB_SHADE_CASE
+    return fail(PTB_E_INVALID, "ptb_scene_shade: unreachable");
+}
+
+extern "C" int ptb_scene_shade(ptb_device* dev, ptb_scene* scene, const ptb_render_params* p, ptb_buffer* rays, int n_rays,
+                               ptb_buffer* radiance, ptb_buffer* stats, ptb_counters* counters) {
+    if (!dev || !scene || !p || !rays || !radiance)
+        return fail(PTB_E_INVALID, "ptb_scene_shade: null device, scene, params, rays or radiance");
+    if (n_rays < 0) return fail(PTB_E_INVALID, "ptb_scene_shade: n_rays %d < 0", n_rays);
+    if (p->mode < 0 || p->mode > PTB_MODE_PATH) return fail(PTB_E_INVALID, "ptb_scene_shade: bad mode %d", p->mode);
+    if (p->max_depth < 1 || p->max_depth > 4096) return fail(PTB_E_INVALID, "ptb_scene_shade: bad max_depth %d", p->max_depth);
+    if (p->mode == PTB_MODE_AO && (p->ao_samples < 1 || p->ao_samples > 4096))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: bad ao_samples %d", p->ao_samples);
+    if (p->accel != PTB_ACCEL_BVH) return fail(PTB_E_INVALID, "ptb_scene_shade: accel %d: only PTB_ACCEL_BVH is available", p->accel);
+    if (p->integrator != PTB_INTEGRATOR_AUTO && p->integrator != PTB_INTEGRATOR_MEGAKERNEL)
+        return fail(PTB_E_INVALID, "ptb_scene_shade: integrator %d: only the megakernel integrator is available", p->integrator);
+    if (scene->dev != dev) return fail(PTB_E_INVALID, "ptb_scene_shade: scene belongs to another device");
+    if (rays->dev != dev || radiance->dev != dev || (stats && stats->dev != dev))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: buffer belongs to another device");
+    if (p->mode == PTB_MODE_DIRECT && (p->light_quad < 0 || p->light_quad >= scene->n_mats))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: light_quad %d out of range", p->light_quad);
+    const size_t n = size_t(n_rays);
+    if (rays->bytes < n * sizeof(ptb_sample_ray))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: rays buffer too small (%zu < %zu)", rays->bytes, n * sizeof(ptb_sample_ray));
+    if (radiance->bytes < n * 16) return fail(PTB_E_INVALID, "ptb_scene_shade: radiance buffer too small (%zu < %zu)", radiance->bytes, n * 16);
+    if (stats && stats->bytes < n * sizeof(ptb_pixel_stats))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: stats buffer too small (%zu < %zu)", stats->bytes, n * sizeof(ptb_pixel_stats));
+    if ((reinterpret_cast<uintptr_t>(rays->d_ptr) & 31u) != 0)
+        return fail(PTB_E_INVALID, "ptb_scene_shade: rays must be 32-byte aligned (one 256-bit load per ray)");
+    if ((reinterpret_cast<uintptr_t>(radiance->d_ptr) & 15u) != 0 || (stats && (reinterpret_cast<uintptr_t>(stats->d_ptr) & 15u) != 0))
+        return fail(PTB_E_INVALID, "ptb_scene_shade: radiance and stats must be 16-byte aligned");
+    if (n_rays == 0) {
+        if (counters) std::memset(counters, 0, sizeof *counters);
+        return PTB_OK;
+    }
+    if (set_device(dev)) return PTB_E_CUDA;
+    const int small = mode_class(scene, p->mode);
+    const ptd::SceneDev sc = scene_dev(scene, small);
+    ptd::ShadeArgs a;
+    std::memset(&a, 0, sizeof a);
+    a.frames_in_batch = 1;
+    a.n_local = n_rays;  // sample slot i = ray i
+    a.max_depth = p->max_depth; a.ao_samples = p->ao_samples; a.ao_max_dist = p->ao_max_dist;
+    if (int rc = setup_light(scene, p, a)) return rc;
+    a.samples = static_cast<float4*>(radiance->d_ptr);
+    a.stats = stats ? static_cast<ptb_pixel_stats*>(stats->d_ptr) : nullptr;
+    a.counters = dev->counters;
+    for (int k = 0; k < 16; ++k) a.tune[k] = dev->tune[k];
+    a.rays = static_cast<const float4*>(rays->d_ptr);
+    if (!dev->cumulative_counters) CU_TRY(cudaMemsetAsync(dev->counters, 0, sizeof(unsigned long long) * ptd::CTR_COUNT, dev->stream));
+    else dev->cumulative_samples += n;
+    const bool st = stats != nullptr;
+    int rc = PTB_OK;
+    switch (p->mode) {
+        case PTB_MODE_PRIMARY: rc = launch_shade_m<PTB_MODE_PRIMARY>(dev, sc, a, small, st); break;
+        case PTB_MODE_AO: rc = launch_shade_m<PTB_MODE_AO>(dev, sc, a, small, st); break;
+        case PTB_MODE_DIRECT: rc = launch_shade_m<PTB_MODE_DIRECT>(dev, sc, a, small, st); break;
+        default: rc = launch_shade_m<PTB_MODE_PATH>(dev, sc, a, small, st); break;
+    }
+    if (rc) return rc;
+    if (counters) {
+        unsigned long long hc[ptd::CTR_COUNT];
+        CU_TRY(cudaMemcpyAsync(hc, dev->counters, sizeof hc, cudaMemcpyDeviceToHost, dev->stream));
+        CU_TRY(cudaStreamSynchronize(dev->stream));
+        std::memset(counters, 0, sizeof *counters);
+        counters->rays_closest = hc[ptd::CTR_CLOSEST]; counters->rays_any = hc[ptd::CTR_ANY];
+        counters->nodes = hc[ptd::CTR_NODES]; counters->tri_tests = hc[ptd::CTR_TESTS];
+        counters->samples = n;
     }
     return PTB_OK;
 }

@@ -133,6 +133,30 @@ struct RenderArgs {
     int tune[16];          // experiment knobs (ptb_device_set_tuning); never change results
 };
 
+// Where the sample of a slot gets its ray and its RNG state (template parameter SRC of k_mega, k_mega_path_regen and path_sm2,
+// which take their arguments as SRC::Args).
+//   CameraRays  ptb_render: slot -> (pixel, frame) -> the reference's camera, GenerateColors.cl:305-310
+//   SampleRays  ptb_scene_shade: record `slot` of the caller's ptb_sample_ray array (o, seed, d, unused), one 256-bit load; the
+//               sample writes samples[slot] and, with statistics, stats[slot] (frames_in_batch = 1, n_local = the ray count)
+struct ShadeArgs : RenderArgs {
+    const float4* rays;  // 2 x float4 per ptb_sample_ray record, 32-byte aligned
+};
+struct CameraRays {
+    static constexpr bool buffer = false;
+    using Args = RenderArgs;
+};
+struct SampleRays {
+    static constexpr bool buffer = true;
+    using Args = ShadeArgs;
+};
+PTD_FI void load_sample_ray(const ShadeArgs& a, long long slot, Ray& r, uint32_t& seed) {
+    float4 o, d;
+    ldg256(a.rays + 2 * (size_t)slot, o, d);
+    r.o = xyz(o);
+    r.d = xyz(d);
+    seed = __float_as_uint(o.w);
+}
+
 template <bool STATS>
 struct SampleStats {
     int tri, quad;
@@ -365,8 +389,8 @@ PTD_FI V3 sample_direct(const Ctx& c, const RenderArgs& a, Ray r, uint32_t& seed
 
 // ---- megakernel: one thread per sample ---------------------------------------------------------
 
-template <int MODE, bool BVH, int SMALL, bool STATS>
-__global__ void __launch_bounds__(128, ((MODE == PTB_MODE_AO || MODE == PTB_MODE_DIRECT) && BVH && SMALL) ? 8 : 0) k_mega(const SceneDev sc, const RenderArgs a) {
+template <int MODE, bool BVH, int SMALL, bool STATS, class SRC = CameraRays>
+__global__ void __launch_bounds__(128, ((MODE == PTB_MODE_AO || MODE == PTB_MODE_DIRECT) && BVH && SMALL) ? 8 : 0) k_mega(const SceneDev sc, const typename SRC::Args a) {
     extern __shared__ __align__(16) unsigned char smem[];
     Ctx c = stage_scene<BVH, SMALL>(sc, smem);
     uint2 lstack_mem[PTD_LSTACK_ENTRIES];
@@ -378,13 +402,22 @@ __global__ void __launch_bounds__(128, ((MODE == PTB_MODE_AO || MODE == PTB_MODE
     QueryStats qs{0u, 0u};
     const bool valid = slot < total;
     if (valid) {
-        const int fi = (int)(slot / a.n_local);
-        const int li = (int)(slot - (long long)fi * a.n_local);
-        const int gid = gid_of_local(a.shard, li);
-        const int frame = a.first_frame + fi;
-        const int gi = gid % a.width, gj = gid / a.width;           // GenerateColors.cl:305-306
-        uint32_t seed = (uint32_t)gid + hash_uint32((uint32_t)frame);  // :308
-        const Ray r = generate_ray(gi, gj, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);   // :310
+        int li, frame;
+        uint32_t seed;
+        Ray r;
+        if constexpr (SRC::buffer) {
+            li = (int)slot;
+            frame = 0;
+            load_sample_ray(a, slot, r, seed);
+        } else {
+            const int fi = (int)(slot / a.n_local);
+            li = (int)(slot - (long long)fi * a.n_local);
+            const int gid = gid_of_local(a.shard, li);
+            frame = a.first_frame + fi;
+            const int gi = gid % a.width, gj = gid / a.width;  // GenerateColors.cl:305-306
+            seed = (uint32_t)gid + hash_uint32((uint32_t)frame);  // :308
+            r = generate_ray(gi, gj, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);   // :310
+        }
         SampleStats<STATS> st{};
         V3 col;
         if (MODE == PTB_MODE_PRIMARY) col = sample_primary<BVH, SMALL, STATS>(c, r, st, rc, qs);
@@ -393,7 +426,7 @@ __global__ void __launch_bounds__(128, ((MODE == PTB_MODE_AO || MODE == PTB_MODE
         else col = trace_rays<BVH, SMALL, STATS>(c, r, seed, a.max_depth, st, rc, qs);  // :312
         a.samples[slot] = make_float4(col.x, col.y, col.z, 1.0f);
         if constexpr (STATS) {
-            if (a.stats && frame == a.stats_frame) {
+            if (a.stats && (SRC::buffer || frame == a.stats_frame)) {
                 uint4* dst = reinterpret_cast<uint4*>(a.stats + li);
                 dst[0] = make_uint4((uint32_t)st.tri, (uint32_t)st.quad, st.t_bits, st.visits_primary);
                 dst[1] = make_uint4(st.visits_secondary, st.count, st.id_hash, qs.tests);
@@ -415,8 +448,8 @@ __global__ void __launch_bounds__(128, ((MODE == PTB_MODE_AO || MODE == PTB_MODE
 // slot from a global counter (one warp-aggregated atomicAdd per refill), so every warp iteration is one
 // path segment for (nearly) 32 live lanes.  Per-sample arithmetic is unchanged -> identical results.
 // COOP (FLAT scenes only): the triangle phase of the query is pooled over the warp (flat_mt_coop)
-template <bool BVH, int SMALL, bool STATS, bool COOP = false>
-__global__ void __launch_bounds__(128, (COOP && !STATS) ? 9 : 0) k_mega_path_regen(const SceneDev sc, const RenderArgs a,
+template <bool BVH, int SMALL, bool STATS, bool COOP = false, class SRC = CameraRays>
+__global__ void __launch_bounds__(128, (COOP && !STATS) ? 9 : 0) k_mega_path_regen(const SceneDev sc, const typename SRC::Args a,
                                                          unsigned long long* work_counter) {
     static_assert(!COOP || (BVH && SMALL == PTD_FLAT), "the pooled triangle phase belongs to the FLAT query");
     extern __shared__ __align__(16) unsigned char smem[];
@@ -450,12 +483,17 @@ __global__ void __launch_bounds__(128, (COOP && !STATS) ? 9 : 0) k_mega_path_reg
                 if (slot >= total) {
                     done = true;
                 } else {
-                    const int fi = (int)(slot / a.n_local);
-                    li = (int)(slot - (long long)fi * a.n_local);
-                    const int gid = gid_of_local(a.shard, li);
-                    frame = a.first_frame + fi;
-                    seed = (uint32_t)gid + hash_uint32((uint32_t)frame);                    // GenerateColors.cl:308
-                    r = generate_ray(gid % a.width, gid / a.width, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);  // :310
+                    if constexpr (SRC::buffer) {
+                        li = (int)slot;
+                        load_sample_ray(a, slot, r, seed);
+                    } else {
+                        const int fi = (int)(slot / a.n_local);
+                        li = (int)(slot - (long long)fi * a.n_local);
+                        const int gid = gid_of_local(a.shard, li);
+                        frame = a.first_frame + fi;
+                        seed = (uint32_t)gid + hash_uint32((uint32_t)frame);                    // GenerateColors.cl:308
+                        r = generate_ray(gid % a.width, gid / a.width, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);  // :310
+                    }
                     radiance = mk(0.f, 0.f, 0.f);
                     mask = mk(1.f, 1.f, 1.f);
                     depth = 0;
@@ -492,7 +530,7 @@ __global__ void __launch_bounds__(128, (COOP && !STATS) ? 9 : 0) k_mega_path_reg
             if (!more || depth >= a.max_depth) {
                 a.samples[slot] = make_float4(cl_max(radiance.x, 0.0f), cl_max(radiance.y, 0.0f), cl_max(radiance.z, 0.0f), 1.0f);  // :260
                 if constexpr (STATS) {
-                    if (a.stats && frame == a.stats_frame) {
+                    if (a.stats && (SRC::buffer || frame == a.stats_frame)) {
                         uint4* dst = reinterpret_cast<uint4*>(a.stats + li);
                         dst[0] = make_uint4((uint32_t)st.tri, (uint32_t)st.quad, st.t_bits, st.visits_primary);
                         dst[1] = make_uint4(st.visits_secondary, st.count, st.id_hash, qs.tests - tests0);
@@ -753,8 +791,9 @@ struct PathCol {
     }
 };
 
-template <bool STATS, int MINB, int NSTEP>
-__global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const RenderArgs a, unsigned long long* work_counter) {
+// The body of k_path_sm2 for either ray source (k_path_sm2: the camera; k_path_sm2_rays: a caller's ptb_sample_ray buffer).
+template <bool STATS, int NSTEP, class SRC>
+PTD_FI void path_sm2(const SceneDev& sc, const typename SRC::Args& a, unsigned long long* work_counter) {
     extern __shared__ __align__(16) unsigned char smem[];
     Ctx c = stage_scene<true, PTD_LARGE>(sc, smem);  // stages nothing (smem_nodes == 0): only the Ctx
     uint2 lstack_mem[PTD_LSTACK_ENTRIES + 1];
@@ -839,7 +878,7 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
                 const V3 radiance = ps.rad();
                 a.samples[PKL(PK_SLOT)] = make_float4(cl_max(radiance.x, 0.0f), cl_max(radiance.y, 0.0f), cl_max(radiance.z, 0.0f), 1.0f);  // :260
                 if constexpr (STATS) {
-                    if (a.stats && frame == a.stats_frame) {
+                    if (a.stats && (SRC::buffer || frame == a.stats_frame)) {
                         uint4* dst = reinterpret_cast<uint4*>(a.stats + li);
                         dst[0] = make_uint4((uint32_t)st.tri, (uint32_t)st.quad, st.t_bits, st.visits_primary);
                         dst[1] = make_uint4(st.visits_secondary, st.count, st.id_hash, qs.tests - tests0);
@@ -865,12 +904,19 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
                 if (slot >= (unsigned long long)total) {
                     state = ST_DONE;
                 } else {
-                    const int fi = (int)(slot / (unsigned)a.n_local);
-                    const int l = (int)(slot - (unsigned long long)fi * (unsigned)a.n_local);
-                    const int gid = gid_of_local(a.shard, l);
-                    li = l; frame = a.first_frame + fi;
-                    uint32_t seed = (uint32_t)gid + hash_uint32((uint32_t)(a.first_frame + fi));  // GenerateColors.cl:308
-                    const Ray r = generate_ray(gid % a.width, gid / a.width, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);  // :310
+                    uint32_t seed;
+                    Ray r;
+                    if constexpr (SRC::buffer) {
+                        li = (int)slot;
+                        load_sample_ray(a, (long long)slot, r, seed);
+                    } else {
+                        const int fi = (int)(slot / (unsigned)a.n_local);
+                        const int l = (int)(slot - (unsigned long long)fi * (unsigned)a.n_local);
+                        const int gid = gid_of_local(a.shard, l);
+                        li = l; frame = a.first_frame + fi;
+                        seed = (uint32_t)gid + hash_uint32((uint32_t)(a.first_frame + fi));  // GenerateColors.cl:308
+                        r = generate_ray(gid % a.width, gid / a.width, CamScale{a.cam_inv_w, a.cam_inv_h, a.cam_aspect}, seed);  // :310
+                    }
                     PKSF(PK_OX, r.o.x); PKSF(PK_OY, r.o.y); PKSF(PK_OZ, r.o.z); PKSF(PK_DX, r.d.x); PKSF(PK_DY, r.d.y); PKSF(PK_DZ, r.d.z);
                     PKSF(PK_RX, 0.0f); PKSF(PK_RY, 0.0f); PKSF(PK_RZ, 0.0f); PKSF(PK_MX, 1.0f); PKSF(PK_MY, 1.0f); PKSF(PK_MZ, 1.0f);
                     PKS(PK_SEED, seed); PKS(PK_SLOT, (uint32_t)slot); PKS(PK_DEPTH, 0);
@@ -892,6 +938,16 @@ __global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const
         flush_counter(a.counters, CTR_NODES, qs.visits);
         flush_counter(a.counters, CTR_TESTS, qs.tests);
     }
+}
+
+template <bool STATS, int MINB, int NSTEP>
+__global__ void __launch_bounds__(128, MINB) k_path_sm2(const SceneDev sc, const RenderArgs a, unsigned long long* work_counter) {
+    path_sm2<STATS, NSTEP, CameraRays>(sc, a, work_counter);
+}
+// ptb_scene_shade: the same kernel on the sample rays of a caller's buffer, under a name of its own (k_path_sm2 keeps its symbol)
+template <bool STATS, int MINB, int NSTEP>
+__global__ void __launch_bounds__(128, MINB) k_path_sm2_rays(const SceneDev sc, const ShadeArgs a, unsigned long long* work_counter) {
+    path_sm2<STATS, NSTEP, SampleRays>(sc, a, work_counter);
 }
 
 // ---- ordered accumulation of a batch: GenerateColors.cl:290-321 --------------------------------
