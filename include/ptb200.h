@@ -132,7 +132,11 @@ int ptb_write_ppm(const char* path, const float* rgba, int width, int height);
 /* ---- resident scene: triangles re-laid out + BVH (BUILD-DEFINED) --------------------- */
 typedef struct ptb_bvh_params {
     int32_t max_leaf;   /* 1..8, default 4 */
-    float pad_rel;      /* child boxes are grown by pad_rel * scene diagonal, default 1e-4 */
+    float pad_rel;      /* child boxes are grown by pad_rel * scene diagonal, default 1e-4.  Must be finite and > 0: 0, negative
+                           and NaN are refused, because without a pad the fp32 boxes of FLAT and 4-wide scenes lose hits
+                           (measured on a planar scene).  The smallest value at which every form still equals the brute-force
+                           loop for ray origins within 100 scene diagonals is 1e-5 on the generated scenes of
+                           tests/test_traversal_scenes.py; at 3e-6 the planar scenes already lose hits (DESIGN.md section 4) */
     int32_t n_bins;     /* SAH bins, default 16 */
     int32_t smem_nodes; /* top-of-tree nodes laid out first (BFS) for shared-memory staging, default 1024 */
     float traverse_cost; /* SAH cost of one node visit relative to one triangle test (<= 0: default 1.2) */

@@ -177,6 +177,9 @@ void make_edge_tris(const ptb_triangle* tris, int n_tris, std::vector<ptb_bvh_tr
 int build_bvh(const ptb_triangle* tris, int n_tris, const ptb_bvh_params& params, BuiltBvh* out) {
     if (!tris || n_tris < 1 || !out) return fail(PTB_E_INVALID, "build_bvh: need at least one triangle");
     if (n_tris >= (1 << 28)) return fail(PTB_E_INVALID, "build_bvh: too many triangles for the leaf encoding");
+    if (!(params.pad_rel > 0.0f) || std::isinf(params.pad_rel))
+        return fail(PTB_E_INVALID, "build_bvh: pad_rel must be a finite number > 0, got %g (without a pad, rounding in the box "
+                    "and triangle tests loses hits)", double(params.pad_rel));
     Builder B;
     B.max_leaf = std::min(std::max(params.max_leaf, 1), PTB_BVH_MAX_LEAF);
     B.n_bins = std::min(std::max(params.n_bins, 2), 256);
@@ -214,7 +217,7 @@ int build_bvh(const ptb_triangle* tris, int n_tris, const ptb_bvh_params& params
     // pad: absolute, relative to the scene diagonal
     const float dx = scene.hi[0] - scene.lo[0], dy = scene.hi[1] - scene.lo[1], dz = scene.hi[2] - scene.lo[2];
     const float diag = std::sqrt(dx * dx + dy * dy + dz * dz);
-    const float pad = std::max(params.pad_rel, 0.0f) * diag;
+    const float pad = params.pad_rel * diag;
 
     // renumber: breadth-first prefix, then depth-first subtrees
     const int n_nodes = int(B.nodes.size());

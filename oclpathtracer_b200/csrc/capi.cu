@@ -522,6 +522,9 @@ extern "C" int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, i
     }
     ptb_bvh_params bp;
     if (bvh_params) bp = *bvh_params; else ptb_bvh_params_default(&bp);
+    if (!(bp.pad_rel > 0.0f) || std::isinf(bp.pad_rel))
+        return fail(PTB_E_INVALID, "ptb_scene_create_gpu: pad_rel must be a finite number > 0, got %g (without a pad, rounding in "
+                    "the box and triangle tests loses hits)", double(bp.pad_rel));
     if (set_device(dev)) return PTB_E_CUDA;
     ptb_scene* s = new ptb_scene();
     s->dev = dev; s->n_tris = n_tris; s->n_mats = n_mats;

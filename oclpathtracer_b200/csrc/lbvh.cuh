@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(256) k_lbvh_finish(const ptb_triangle* tris, c
     const float dx = ordered_to_float(scene_bounds[3]) - ordered_to_float(scene_bounds[0]);
     const float dy = ordered_to_float(scene_bounds[4]) - ordered_to_float(scene_bounds[1]);
     const float dz = ordered_to_float(scene_bounds[5]) - ordered_to_float(scene_bounds[2]);
-    const float pad = fmaxf(pad_rel, 0.0f) * sqrtf(dx * dx + dy * dy + dz * dz);
+    const float pad = pad_rel * sqrtf(dx * dx + dy * dy + dz * dz);  // pad_rel > 0: checked by ptb_scene_create_gpu
     if (i < n - 1) {
         float4* nd = nodes + 4 * (size_t)i;
         // padded [lo, hi] of each child -> centre / half-extent widened by two ulps (same rule as the host builder)
