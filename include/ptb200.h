@@ -158,6 +158,18 @@ int ptb_scene_create(ptb_device* dev, const ptb_triangle* tris, int n_tris, cons
  * triangles instead of seconds; lower tree quality than the host SAH build.  Needs >= 2 triangles.          */
 int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, int n_tris, const ptb_material* mats, int n_mats,
                          const ptb_bvh_params* bvh_params /* NULL = default */, ptb_scene** out);
+/* The same scene from records that already live on the device (triangles a torch pipeline made or deformed): tris holds n_tris
+ * ptb_triangle and mats n_mats ptb_material records (64 bytes each, 16-byte aligned; a ptb_buffer_create buffer or a tensor's
+ * storage through ptb_buffer_wrap, both of `dev`).  The tree, node bytes, tri_order, quantised nodes, grid, ptb_scene_info and
+ * every render, intersect and shade result equal ptb_scene_create_gpu's for the same records.  bvh_params: max_leaf and pad_rel
+ * apply; force_width must be 0 or 2 (the FLAT and 4-wide forms need the host builder).  Needs 2 <= n_tris < 2^28 and
+ * n_mats >= 1.  The records are checked on the device as ptb_scene_create_gpu checks them on the host (every id in
+ * [0, n_mats); every vertex float, w included, |v| <= 3e38), and the message names the lowest offending triangle.  Read on
+ * the device's stream, so a device made with ptb_device_create_on_stream on torch's current stream sees the work that wrote
+ * them; synchronises and returns when the scene is ready.  The scene keeps its own copies: the caller may overwrite or free
+ * tris and mats at once.                                                                                                    */
+int ptb_scene_create_from_device(ptb_device* dev, ptb_buffer* tris, int n_tris, ptb_buffer* mats, int n_mats,
+                                 const ptb_bvh_params* bvh_params /* NULL = default */, ptb_scene** out);
 int ptb_scene_destroy(ptb_scene* scene);
 int ptb_scene_info(ptb_scene* scene, int* n_nodes, int* n_tris, int* depth, int* smem_nodes);
 /* form of the resident scene: 1 (FLAT: ptb_bvh_leafbox records, scenes of <= 32 leaves and <= 64 triangles), 4

@@ -104,7 +104,7 @@ EXPORTS = [
     "ptb_buffer_map", "ptb_buffer_unmap", "ptb_buffer_clear", "ptb_buffer_device_ptr", "ptb_buffer_mark_dirty", "ptb_buffer_size",
     "ptb_kernel_get", "ptb_kernel_set_int", "ptb_launch1d", "ptb_launch_serialize", "ptb_launch_deserialize", "ptb_load_model", "ptb_tessellate",
     "ptb_light_from_quad", "ptb_free", "ptb_to_rgb8", "ptb_write_ppm", "ptb_bvh_params_default",
-    "ptb_bvh_build_host", "ptb_scene_create", "ptb_scene_create_gpu", "ptb_scene_destroy", "ptb_scene_info", "ptb_scene_bvh_width", "ptb_scene_mode_width", "ptb_scene_copy_bvh", "ptb_scene_copy_bvh_quantized",
+    "ptb_bvh_build_host", "ptb_scene_create", "ptb_scene_create_gpu", "ptb_scene_create_from_device", "ptb_scene_destroy", "ptb_scene_info", "ptb_scene_bvh_width", "ptb_scene_mode_width", "ptb_scene_copy_bvh", "ptb_scene_copy_bvh_quantized",
     "ptb_render_params_default", "ptb_render_local_pixels", "ptb_render", "ptb_render_host",
     "ptb_buffer_ipc_export", "ptb_buffer_ipc_import", "ptb_render_gather",
     "ptb_render_host_async", "ptb_job_wait", "ptb_host_alloc", "ptb_host_free", "ptb_trace", "ptb_scene_intersect", "ptb_scene_shade",
@@ -157,6 +157,7 @@ def lib():
         L.ptb_buffer_to_rgb8.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.ptb_scene_create.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.ptb_scene_create_gpu.argtypes = L.ptb_scene_create.argtypes
+        L.ptb_scene_create_from_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.ptb_scene_info.argtypes = [C.c_void_p] + [C.c_void_p] * 4
         L.ptb_scene_copy_bvh.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.ptb_render.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -371,6 +372,15 @@ class Device:
     def scene(self, tris, mats, bvh_params=None, gpu_build=False):
         return Scene(self, tris, mats, bvh_params, gpu_build)
 
+    def scene_from_device(self, tris, mats, bvh_params=None):
+        """ptb_scene_create_from_device: the scene Device.scene(..., gpu_build=True) builds, from records already on this device.
+
+        tris is a Buffer of TRIANGLE_DTYPE records or a contiguous CUDA tensor of shape (n, 16) with 4-byte elements (float32
+        records; the id is the int32 bits of column 12); mats is a Buffer, an (n_mats, 16) CUDA tensor or a numpy MATERIAL_DTYPE
+        array (uploaded through a temporary Buffer).  With tensors the Device must have been created on torch's current stream,
+        so that the build reads the records after the work that wrote them.  Synchronises; the scene keeps its own copies."""
+        return Scene(self, tris, mats, bvh_params, from_device=True)
+
     def close(self):
         if self._h:
             for c in list(self._children):
@@ -582,7 +592,8 @@ class Device:
 
 
 class _CallArgs:
-    """Buffers or CUDA torch tensors as ptb_buffer handles for one call of `what` (Device.intersect, Device.shade).
+    """Buffers or CUDA torch tensors as ptb_buffer handles for one call of `what` (Device.intersect, Device.shade,
+    Device.scene_from_device).
 
     Tensors must be contiguous CUDA tensors of 4-byte elements, and the Device must have been created on torch's current
     stream: on another stream the call would race with the work that wrote its inputs.  Used as a context manager, the
@@ -693,15 +704,44 @@ class Buffer:
 class Scene:
     """Resident scene: relaid triangles + BVH (BUILD-DEFINED; the reference is brute force)."""
 
-    def __init__(self, dev, tris, mats, bvh_params=None, gpu_build=False):
+    def __init__(self, dev, tris, mats, bvh_params=None, gpu_build=False, from_device=False):
         self.dev = dev
         self._h = C.c_void_p()
-        tris = np.ascontiguousarray(tris)
-        mats = np.ascontiguousarray(mats)
-        create = lib().ptb_scene_create_gpu if gpu_build else lib().ptb_scene_create
-        _check(create(dev._h, _p(tris), len(tris), _p(mats), len(mats),
-                                      C.byref(bvh_params) if bvh_params is not None else None, C.byref(self._h)))
+        bp = C.byref(bvh_params) if bvh_params is not None else None
+        if from_device:
+            self._create_from_device(tris, mats, bp)
+        else:
+            tris = np.ascontiguousarray(tris)
+            mats = np.ascontiguousarray(mats)
+            create = lib().ptb_scene_create_gpu if gpu_build else lib().ptb_scene_create
+            _check(create(dev._h, _p(tris), len(tris), _p(mats), len(mats), bp, C.byref(self._h)))
         dev._children.append(self)
+
+    def _create_from_device(self, tris, mats, bp):
+        def count(x, name):
+            if isinstance(x, Buffer):
+                return x.nbytes // 64
+            if not hasattr(x, "is_cuda") or x.dim() != 2 or x.shape[1] != 16:
+                raise PtbError(f"Device.scene_from_device: {name} is a Buffer or a CUDA tensor of shape (n, 16), got "
+                               f"{type(x).__name__} {tuple(getattr(x, 'shape', ()))}")
+            return x.shape[0]
+
+        staged = None
+        if isinstance(mats, np.ndarray):
+            if mats.dtype != MATERIAL_DTYPE:
+                raise PtbError(f"Device.scene_from_device: a numpy mats array has MATERIAL_DTYPE, got {mats.dtype}")
+            staged = Buffer(self.dev, mats.nbytes)
+            if len(mats):
+                staged.write(mats)
+            mats = staged
+        try:
+            n_tris, n_mats = count(tris, "tris"), count(mats, "mats")
+            with _CallArgs(self.dev, "Device.scene_from_device", tris, mats) as args:
+                _check(lib().ptb_scene_create_from_device(self.dev._h, args.handle(tris), n_tris, args.handle(mats), n_mats, bp,
+                                                          C.byref(self._h)))
+        finally:
+            if staged is not None:
+                staged.close()
 
     def info(self):
         a, b, c, d = C.c_int(), C.c_int(), C.c_int(), C.c_int()

@@ -139,8 +139,9 @@ struct ptb_scene {
     int n_nodes = 0, depth = 0, bfs_nodes = 0;
     int* d_order = nullptr;               // GPU-built scenes: BVH position -> caller index (device)
     bool host_copy_valid = true;          // false until a GPU-built tree has been downloaded
-    std::vector<ptb_triangle> host_tris;  // kept for the default light lookup and for copies of the scene on helper devices
+    std::vector<ptb_triangle> host_tris;  // host-built scenes: the default light lookup and copies of the scene on helper devices
     std::vector<ptb_material> host_mats;
+    std::vector<ptd::SceneLight> lights;  // device-built scenes: the light of each quad id in [0, n_mats) (setup_light)
 };
 
 static int set_device(ptb_device* dev) {
@@ -506,13 +507,67 @@ extern "C" int ptb_scene_create(ptb_device* dev, const ptb_triangle* tris, int n
     return scene_create_impl(dev, tris, n_tris, mats, n_mats, bvh_params, nullptr, out);
 }
 
-// Scene whose BVH is built on the device (lbvh.cuh).  Only the root is guaranteed to sit at index 0, so one
-// node is staged in shared memory; everything else is traversed from L2/HBM.
+static int check_pad_rel(const char* what, const ptb_bvh_params& bp) {
+    if (!(bp.pad_rel > 0.0f) || std::isinf(bp.pad_rel))
+        return fail(PTB_E_INVALID, "%s: pad_rel must be a finite number > 0, got %g (without a pad, rounding in "
+                    "the box and triangle tests loses hits)", what, double(bp.pad_rel));
+    return PTB_OK;
+}
+
+// The device half of both LBVH constructors (lbvh.cuh).  From n_tris caller-order triangle and n_mats material records on the
+// device (read on dev->stream and not kept): the validation verdicts, the caller-order edge triangles, the packed materials,
+// the light table, the tree and its quantised encoding.  The verdicts and the light table come back in the synchronisation
+// that fetches the tree depth; records that fail validation leave no scene.  Only the root is guaranteed to sit at index 0, so
+// one node is staged in shared memory; everything else is traversed from L2/HBM.
+static int scene_create_lbvh(ptb_device* dev, const char* what, const ptb_triangle* d_tris, int n_tris, const ptb_material* d_mats,
+                             int n_mats, const ptb_bvh_params& bp, ptb_scene** out) {
+    ptb_scene* s = new ptb_scene();
+    s->dev = dev; s->n_tris = n_tris; s->n_mats = n_mats;
+    s->host_copy_valid = false;
+    s->n_nodes = n_tris - 1; s->bfs_nodes = 1; s->small = false; s->width = 2;
+    const size_t light_bytes = sizeof(ptd::SceneLight) * size_t(n_mats);
+    std::vector<unsigned char> check(16 + light_bytes);  // the two verdicts (k_scene_tris), then the light table
+    unsigned long long* d_check = nullptr;
+    auto fail_out = [&](int code) { if (d_check) cudaFree(d_check); ptb_scene_destroy(s); return code; };
+    if (cudaMalloc((void**)&s->d_tris_orig, size_t(n_tris) * 48) != cudaSuccess || cudaMalloc((void**)&s->d_mats, size_t(n_mats) * 32) != cudaSuccess ||
+        cudaMalloc((void**)&d_check, check.size()) != cudaSuccess)
+        return fail_out(fail(PTB_E_NOMEM, "%s: cudaMalloc failed", what));
+    ptd::SceneLight* d_lights = reinterpret_cast<ptd::SceneLight*>(d_check + 2);
+    const unsigned grid_t = unsigned((n_tris + 255) / 256), grid_m = unsigned((n_mats + 255) / 256);
+    if (cudaMemsetAsync(d_check, 0xff, 16, dev->stream) != cudaSuccess || cudaMemsetAsync(d_lights, 0x7f, light_bytes, dev->stream) != cudaSuccess)
+        return fail_out(fail(PTB_E_CUDA, "%s: cudaMemsetAsync failed", what));
+    ptd::k_scene_tris<<<grid_t, 256, 0, dev->stream>>>(d_tris, n_tris, n_mats, d_check, s->d_tris_orig, d_lights);
+    ptd::k_scene_mats<<<grid_m, 256, 0, dev->stream>>>(d_mats, n_mats, s->d_mats);
+    ptd::k_scene_lights<<<grid_m, 256, 0, dev->stream>>>(d_tris, n_tris, n_mats, d_lights);
+    if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) return fail_out(fail(PTB_E_CUDA, "%s: launch failed: %s", what, cudaGetErrorString(e)));
+    if (int rc = ptd::build_lbvh_device(dev->stream, d_tris, n_tris, bp.max_leaf, bp.pad_rel, &s->d_nodes, &s->d_tris, &s->d_order, &s->depth,
+                                        d_check, check.data(), check.size()))
+        return fail_out(rc);
+    unsigned long long bad[2];
+    std::memcpy(bad, check.data(), sizeof bad);
+    if (bad[0] != ~0ull || bad[1] != ~0ull) {  // the lowest offending index; on a tie the id is reported, as the host loop does
+        const unsigned long long first_id = bad[0] >> 32;
+        if (first_id <= bad[1])
+            return fail_out(fail(PTB_E_INVALID, "%s: triangle %d has id %d outside [0,%d)", what, int(first_id), int(uint32_t(bad[0])), n_mats));
+        return fail_out(fail(PTB_E_INVALID, "%s: triangle %d has a non-finite vertex", what, int(bad[1])));
+    }
+    s->lights.resize(size_t(n_mats));
+    std::memcpy(s->lights.data(), check.data() + 16, light_bytes);
+    cudaFree(d_check); d_check = nullptr;
+    if (int rc = quantize_scene(s)) return fail_out(rc);
+    *out = s;
+    return PTB_OK;
+}
+
+// Scene whose BVH is built on the device from host records: checked here, uploaded, then built as ptb_scene_create_from_device
+// builds it.
 extern "C" int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, int n_tris, const ptb_material* mats,
                                     int n_mats, const ptb_bvh_params* bvh_params, ptb_scene** out) {
     if (!dev || !tris || !mats || !out || n_tris < 2 || n_mats < 1)
         return fail(PTB_E_INVALID, "ptb_scene_create_gpu: bad arguments (needs >= 2 triangles)");
     *out = nullptr;
+    if (n_tris >= (1 << 28))  // a leaf reference holds first << 3 in 32 bits
+        return fail(PTB_E_INVALID, "ptb_scene_create_gpu: %d triangles; the leaf encoding holds fewer than 2^28", n_tris);
     for (int i = 0; i < n_tris; ++i) {
         if (tris[i].id < 0 || tris[i].id >= n_mats)
             return fail(PTB_E_INVALID, "ptb_scene_create_gpu: triangle %d has id %d outside [0,%d)", i, tris[i].id, n_mats);
@@ -522,44 +577,48 @@ extern "C" int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, i
     }
     ptb_bvh_params bp;
     if (bvh_params) bp = *bvh_params; else ptb_bvh_params_default(&bp);
-    if (!(bp.pad_rel > 0.0f) || std::isinf(bp.pad_rel))
-        return fail(PTB_E_INVALID, "ptb_scene_create_gpu: pad_rel must be a finite number > 0, got %g (without a pad, rounding in "
-                    "the box and triangle tests loses hits)", double(bp.pad_rel));
+    if (int rc = check_pad_rel("ptb_scene_create_gpu", bp)) return rc;
     if (set_device(dev)) return PTB_E_CUDA;
-    ptb_scene* s = new ptb_scene();
-    s->dev = dev; s->n_tris = n_tris; s->n_mats = n_mats;
-    s->host_tris.assign(tris, tris + n_tris);
-    s->host_copy_valid = false;
-    std::vector<ptb_bvh_tri> orig;
-    make_edge_tris(tris, n_tris, &orig);
-    std::vector<float4> m(size_t(n_mats) * 2);
-    for (int i = 0; i < n_mats; ++i) {
-        m[2 * i] = make_float4(mats[i].albedo.x, mats[i].albedo.y, mats[i].albedo.z, mats[i].roughness);
-        float tbits;
-        std::memcpy(&tbits, &mats[i].type, 4);
-        m[2 * i + 1] = make_float4(mats[i].emissive.x, mats[i].emissive.y, mats[i].emissive.z, tbits);
-    }
-    ptb_triangle* d_raw = nullptr;
+    ptb_triangle* d_raw = nullptr;  // the triangle records, then the material records
+    if (cudaMalloc((void**)&d_raw, (size_t(n_tris) + size_t(n_mats)) * 64) != cudaSuccess)
+        return fail(PTB_E_NOMEM, "ptb_scene_create_gpu: cudaMalloc failed");
+    ptb_material* d_rawm = reinterpret_cast<ptb_material*>(d_raw + n_tris);
     int rc = PTB_OK;
-    auto fail_out = [&](int code) { if (d_raw) cudaFree(d_raw); ptb_scene_destroy(s); return code; };
-    if (cudaMalloc((void**)&d_raw, size_t(n_tris) * 64) != cudaSuccess) return fail_out(fail(PTB_E_NOMEM, "ptb_scene_create_gpu: cudaMalloc failed"));
-    if (cudaMemcpyAsync(d_raw, tris, size_t(n_tris) * 64, cudaMemcpyHostToDevice, dev->stream) != cudaSuccess)
-        return fail_out(fail(PTB_E_CUDA, "ptb_scene_create_gpu: upload failed"));
-    float4* d_nodes = nullptr; float4* d_otris = nullptr; int* d_order = nullptr; int depth = 0;
-    if ((rc = ptd::build_lbvh_device(dev->stream, d_raw, n_tris, bp.max_leaf, bp.pad_rel, &d_nodes, &d_otris, &d_order, &depth))) return fail_out(rc);
-    s->d_nodes = d_nodes; s->d_tris = d_otris; s->d_order = d_order;
-    s->n_nodes = n_tris - 1; s->depth = depth; s->bfs_nodes = 1; s->small = false; s->width = 2;
-    auto up = [&](float4** d, const void* h, size_t bytes) -> int {
-        CU_TRY(cudaMalloc((void**)d, bytes));
-        CU_TRY(cudaMemcpyAsync(*d, h, bytes, cudaMemcpyHostToDevice, dev->stream));
-        return PTB_OK;
-    };
-    if ((rc = up(&s->d_tris_orig, orig.data(), orig.size() * 48)) || (rc = up(&s->d_mats, m.data(), m.size() * 16))) return fail_out(rc);
-    if (cudaStreamSynchronize(dev->stream) != cudaSuccess) return fail_out(fail(PTB_E_CUDA, "ptb_scene_create_gpu: sync failed"));
-    if ((rc = quantize_scene(s))) return fail_out(rc);
+    if (cudaMemcpyAsync(d_raw, tris, size_t(n_tris) * 64, cudaMemcpyHostToDevice, dev->stream) != cudaSuccess ||
+        cudaMemcpyAsync(d_rawm, mats, size_t(n_mats) * 64, cudaMemcpyHostToDevice, dev->stream) != cudaSuccess) {
+        cudaStreamSynchronize(dev->stream);
+        rc = fail(PTB_E_CUDA, "ptb_scene_create_gpu: upload failed");
+    } else {
+        rc = scene_create_lbvh(dev, "ptb_scene_create_gpu", d_raw, n_tris, d_rawm, n_mats, bp, out);
+    }
     cudaFree(d_raw);
-    *out = s;
-    return PTB_OK;
+    return rc;
+}
+
+extern "C" int ptb_scene_create_from_device(ptb_device* dev, ptb_buffer* tris, int n_tris, ptb_buffer* mats, int n_mats,
+                                            const ptb_bvh_params* bvh_params, ptb_scene** out) {
+    if (!dev || !tris || !mats || !out) return fail(PTB_E_INVALID, "ptb_scene_create_from_device: null device, tris, mats or out");
+    *out = nullptr;
+    if (n_tris < 2 || n_mats < 1)
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: needs >= 2 triangles and >= 1 material, got %d and %d", n_tris, n_mats);
+    if (n_tris >= (1 << 28))  // before the sizes: nothing is read
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: %d triangles; the leaf encoding holds fewer than 2^28", n_tris);
+    if (tris->dev != dev || mats->dev != dev) return fail(PTB_E_INVALID, "ptb_scene_create_from_device: buffer belongs to another device");
+    if (tris->bytes < size_t(n_tris) * 64)
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: tris buffer too small (%zu < %zu)", tris->bytes, size_t(n_tris) * 64);
+    if (mats->bytes < size_t(n_mats) * 64)
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: mats buffer too small (%zu < %zu)", mats->bytes, size_t(n_mats) * 64);
+    if (((reinterpret_cast<uintptr_t>(tris->d_ptr) | reinterpret_cast<uintptr_t>(mats->d_ptr)) & 15u) != 0)
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: tris and mats must be 16-byte aligned (float4 loads)");
+    ptb_bvh_params bp;
+    if (bvh_params) bp = *bvh_params; else ptb_bvh_params_default(&bp);
+    if (int rc = check_pad_rel("ptb_scene_create_from_device", bp)) return rc;
+    if (bp.force_width != 0 && bp.force_width != 2)
+        return fail(PTB_E_INVALID, "ptb_scene_create_from_device: force_width = %d; only the binary form (0 or 2) is built on the device",
+                    bp.force_width);
+    if (set_device(dev)) return PTB_E_CUDA;
+    return scene_create_lbvh(dev, "ptb_scene_create_from_device", static_cast<const ptb_triangle*>(tris->d_ptr), n_tris,
+                             static_cast<const ptb_material*>(mats->d_ptr), n_mats, bp, out);
 }
 
 extern "C" int ptb_bvh_build_host(const ptb_triangle* tris, int n_tris, const ptb_bvh_params* bvh_params, int width,
@@ -873,6 +932,12 @@ static int setup_light(const ptb_scene* scene, const ptb_render_params* p, ptd::
     const bool have_light = p->light_ea[0] != 0.f || p->light_ea[1] != 0.f || p->light_ea[2] != 0.f;
     if (have_light) {
         std::memcpy(a.light_p1, p->light_p1, 12); std::memcpy(a.light_ea, p->light_ea, 12); std::memcpy(a.light_eb, p->light_eb, 12);
+    } else if (p->mode == PTB_MODE_DIRECT && !scene->lights.empty()) {  // device-built scene: its light table (k_scene_lights)
+        const int q = p->light_quad;
+        if (q < 0 || q >= scene->n_mats || scene->lights[size_t(q)].q >= scene->n_tris)
+            return fail(PTB_E_NOTFOUND, "ptb_light_from_quad: no triangle pair with id %d", q);
+        const ptd::SceneLight& L = scene->lights[size_t(q)];
+        std::memcpy(a.light_p1, L.p1, 12); std::memcpy(a.light_ea, L.ea, 12); std::memcpy(a.light_eb, L.eb, 12);
     } else if (p->mode == PTB_MODE_DIRECT) {
         if (int rc = ptb_light_from_quad(scene->host_tris.data(), scene->n_tris, p->light_quad, a.light_p1, a.light_ea, a.light_eb)) return rc;
     }

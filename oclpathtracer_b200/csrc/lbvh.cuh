@@ -9,6 +9,8 @@
 //   k_lbvh_fit          bottom-up: one thread per sorted triangle climbs to the root; the second arrival at a
 //                       node (atomic flag) unions the two child boxes and goes on
 //   k_lbvh_finish       pad the boxes, write the precomputed-edge triangle records in sorted order
+//   k_scene_tris / _mats / _lights   the rest of the scene from the caller-order records: validation verdicts, edge
+//                       triangles in caller order, packed materials, the light of every quad id
 //
 // The result is deterministic (unique sort keys, exact min/max) and equivalent to the brute-force loop by the
 // same argument as the host SAH builder: every stored box is the exact bound of its triangles plus the pad.
@@ -128,10 +130,9 @@ __global__ void __launch_bounds__(256) k_lbvh_fit(const unsigned long long* keys
     const int tri = (int)(keys[k] & 0xffffffffull);
     float4 lo = tlo[tri], hi = thi[tri];
     int p = parent[(n - 1) + k];
-    int depth = 0;
+    int depth = 0;  // internal nodes on the longest path down from the subtree this thread carries (0 at a leaf)
     while (p >= 0) {
         const int node = p >> 1, side = p & 1;
-        ++depth;
         float4* nd = nodes + 4 * (size_t)node;
         // keep the child reference stored in .w of words 0/1
         if (side == 0) {
@@ -142,7 +143,11 @@ __global__ void __launch_bounds__(256) k_lbvh_fit(const unsigned long long* keys
             nd[3] = make_float4(hi.x, hi.y, hi.z, 0.f);
         }
         __threadfence();
-        if (atomicAdd(&flags[node], 1) == 0) return;  // the sibling subtree is not finished yet
+        // the first arrival leaves its subtree's depth + 1 and stops (the sibling subtree is not finished yet); the second
+        // takes the deeper of the two, so the root gets the tree's depth whichever leaves' threads climb to it
+        const int sibling = atomicAdd(&flags[node], depth + 1);
+        if (sibling == 0) return;
+        depth = 1 + max(depth, sibling - 1);
         __threadfence();
         const float4 a0 = __ldcg(nd), a1 = __ldcg(nd + 1), b0 = __ldcg(nd + 2), b1 = __ldcg(nd + 3);  // L2, not a stale L1 line
         lo = make_float4(fminf(a0.x, b0.x), fminf(a0.y, b0.y), fminf(a0.z, b0.z), 0.f);
@@ -158,7 +163,7 @@ __global__ void __launch_bounds__(256) k_lbvh_finish(const ptb_triangle* tris, c
     const float dx = ordered_to_float(scene_bounds[3]) - ordered_to_float(scene_bounds[0]);
     const float dy = ordered_to_float(scene_bounds[4]) - ordered_to_float(scene_bounds[1]);
     const float dz = ordered_to_float(scene_bounds[5]) - ordered_to_float(scene_bounds[2]);
-    const float pad = pad_rel * sqrtf(dx * dx + dy * dy + dz * dz);  // pad_rel > 0: checked by ptb_scene_create_gpu
+    const float pad = pad_rel * sqrtf(dx * dx + dy * dy + dz * dz);  // pad_rel > 0: checked by the scene constructors
     if (i < n - 1) {
         float4* nd = nodes + 4 * (size_t)i;
         // padded [lo, hi] of each child -> centre / half-extent widened by two ulps (same rule as the host builder)
@@ -187,15 +192,84 @@ __global__ void __launch_bounds__(256) k_lbvh_finish(const ptb_triangle* tris, c
     }
 }
 
+// ---- the rest of a device-built scene, from the caller-order records on the device ------------------------------------
+// (ptb_scene_create_gpu, ptb_scene_create_from_device).  Every output is a bit copy or a plain fp32 subtraction of the records,
+// so it equals what the host computes from the same records (make_edge_tris, the material packing of scene_create_impl,
+// ptb_light_from_quad).
+
+// The area light of one quad id as ptb_light_from_quad derives it; q = the first even triangle index with q + 1 < n and
+// id == quad, or a value >= n when there is no such pair (the table starts as 0x7f bytes).
+struct SceneLight {
+    int32_t q;
+    float p1[3], ea[3], eb[3];
+};
+static_assert(sizeof(SceneLight) == 40, "SceneLight is read back as 40-byte records");
+
+// One thread per triangle: the validation verdicts (bad[0]: the lowest index whose id is outside [0, n_mats), as
+// index << 32 | id bits; bad[1]: the lowest index with a vertex float failing |v| <= 3e38, w included; both start all ones),
+// the caller-order edge triangle (edge_tri: index = i, quad = id, pad = 0) and the first even q of each quad id.
+__global__ void __launch_bounds__(256) k_scene_tris(const ptb_triangle* tris, int n, int n_mats, unsigned long long* bad,
+                                                    float4* otris, SceneLight* lights) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    bool bad_id = false, bad_v = false;
+    int id = -1;
+    if (i < n) {
+        const float4* p = reinterpret_cast<const float4*>(tris + i);
+        const float4 a = p[0], b = p[1], c = p[2];
+        id = reinterpret_cast<const int*>(tris + i)[12];
+        bad_id = id < 0 || id >= n_mats;
+        const float v[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+        for (int k = 0; k < 12; ++k) bad_v |= !(fabsf(v[k]) <= 3.0e38f);
+        otris[3 * (size_t)i + 0] = make_float4(a.x, a.y, a.z, __int_as_float(i));
+        otris[3 * (size_t)i + 1] = make_float4(b.x - a.x, b.y - a.y, b.z - a.z, __int_as_float(id));  // GenerateColors.cl:92
+        otris[3 * (size_t)i + 2] = make_float4(c.x - a.x, c.y - a.y, c.z - a.z, 0.f);                  // GenerateColors.cl:93
+    }
+    // lanes hold consecutive indices: the lowest offending lane of a warp has the warp's lowest index, one atomic per warp
+    const unsigned mid = __ballot_sync(0xffffffffu, bad_id), mv = __ballot_sync(0xffffffffu, bad_v);
+    if (mid && lane == __ffs(mid) - 1) atomicMin(&bad[0], ((unsigned long long)i << 32) | (unsigned int)id);
+    if (mv && lane == __ffs(mv) - 1) atomicMin(&bad[1], (unsigned long long)i);
+    // light pairs: lanes of one id meet in one atomic (tessellated scenes hold long runs of one id)
+    const int key = (i < n && (i & 1) == 0 && i + 1 < n && !bad_id) ? id : -1;
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    if (key >= 0 && lane == __ffs(peers) - 1) atomicMin(&lights[key].q, i);
+}
+
+// one thread per material: the two float4s the kernels read (albedo.xyz, roughness | emissive.xyz, bits of type)
+__global__ void __launch_bounds__(256) k_scene_mats(const ptb_material* mats, int n_mats, float4* out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_mats) return;
+    const float4* p = reinterpret_cast<const float4*>(mats + i);
+    const float4 albedo = p[0], emissive = p[1], rt = p[2];  // rt.x = roughness, rt.y = type
+    out[2 * (size_t)i] = make_float4(albedo.x, albedo.y, albedo.z, rt.x);
+    out[2 * (size_t)i + 1] = make_float4(emissive.x, emissive.y, emissive.z, rt.y);
+}
+
+// one thread per quad id, after k_scene_tris: p1 = tris[q].p1, ea = tris[q].p2 - p1, eb = tris[q + 1].p2 - p1
+__global__ void __launch_bounds__(256) k_scene_lights(const ptb_triangle* tris, int n, int n_mats, SceneLight* lights) {
+    const int quad = blockIdx.x * blockDim.x + threadIdx.x;
+    if (quad >= n_mats) return;
+    SceneLight& L = lights[quad];
+    const int q = L.q;
+    if (q >= n) return;
+    const float4 a = reinterpret_cast<const float4*>(tris + q)[0], b = reinterpret_cast<const float4*>(tris + q)[1];
+    const float4 d = reinterpret_cast<const float4*>(tris + q + 1)[1];
+    L.p1[0] = a.x; L.p1[1] = a.y; L.p1[2] = a.z;
+    L.ea[0] = b.x - a.x; L.ea[1] = b.y - a.y; L.ea[2] = b.z - a.z;
+    L.eb[0] = d.x - a.x; L.eb[1] = d.y - a.y; L.eb[2] = d.z - a.z;
+}
+
 #define LBVH_TRY(expr)                                                                                       \
     do {                                                                                                     \
         cudaError_t e__ = (expr);                                                                            \
         if (e__ != cudaSuccess) { rc = ptb::fail(PTB_E_CUDA, "%s failed: %s", #expr, cudaGetErrorString(e__)); goto cleanup; } \
     } while (0)
 
-// d_tris: n caller-order records on the device.  Outputs are cudaMalloc'd here (caller frees).
+// d_tris: n caller-order records on the device.  Outputs are cudaMalloc'd here (caller frees).  The `readback` bytes at
+// d_readback (work the caller enqueued before on `st`) are copied to h_readback in the same synchronisation as the depth.
 static int build_lbvh_device(cudaStream_t st, const ptb_triangle* d_tris, int n, int max_leaf, float pad_rel, float4** d_nodes_out,
-                             float4** d_otris_out, int** d_order_out, int* depth_out) {
+                             float4** d_otris_out, int** d_order_out, int* depth_out, const void* d_readback, void* h_readback,
+                             size_t readback) {
     int rc = PTB_OK;
     float4 *tlo = nullptr, *thi = nullptr, *nodes = nullptr, *otris = nullptr;
     unsigned long long *keys = nullptr, *keys_sorted = nullptr;
@@ -231,6 +305,7 @@ static int build_lbvh_device(cudaStream_t st, const ptb_triangle* d_tris, int n,
     k_lbvh_finish<<<grid_n, 256, 0, st>>>(d_tris, keys_sorted, n, pad_rel, misc, nodes, otris, order);
     LBVH_TRY(cudaGetLastError());
     LBVH_TRY(cudaMemcpyAsync(&depth, misc + 6, 4, cudaMemcpyDeviceToHost, st));
+    if (readback) LBVH_TRY(cudaMemcpyAsync(h_readback, d_readback, readback, cudaMemcpyDeviceToHost, st));
     LBVH_TRY(cudaStreamSynchronize(st));
     *d_nodes_out = nodes; *d_otris_out = otris; *d_order_out = order; *depth_out = depth;
     nodes = nullptr; otris = nullptr; order = nullptr;
