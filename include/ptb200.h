@@ -142,8 +142,16 @@ typedef struct ptb_bvh_params {
     float traverse_cost; /* SAH cost of one node visit relative to one triangle test (<= 0: default 1.2) */
     int32_t force_width; /* 0 = pick the scene class (below); 1 | 4 | 2 = force the FLAT / 4-wide / binary form (A/B runs and tests;
                             ptb_scene_create fails when the scene does not qualify for the forced form) */
-    int32_t reserved[2];
+    int32_t builder;    /* the tree the device entry points (ptb_scene_create_gpu, ptb_scene_create_from_device) build:
+                           PTB_BUILDER_LBVH (default; max_leaf and pad_rel apply) or PTB_BUILDER_SAH: on the device, the tree
+                           ptb_scene_create(force_width = 2) builds on the host from the same records, byte for byte (nodes,
+                           tri_order, ptb_scene_info, quantised nodes, so every render, intersect and shade result); max_leaf,
+                           pad_rel, n_bins, smem_nodes and traverse_cost apply as on the host.  Other values are refused.  The host
+                           entry points (ptb_scene_create, ptb_bvh_build_host) have one builder and ignore the field. */
+    int32_t reserved[1];
 } ptb_bvh_params;
+#define PTB_BUILDER_LBVH 0 /* Morton-order LBVH (csrc/lbvh.cuh): the fastest build, more node visits per ray */
+#define PTB_BUILDER_SAH 1  /* the host's binned-SAH tree, built on the device (csrc/sah_build.cuh) */
 void ptb_bvh_params_default(ptb_bvh_params* p);
 
 /* host-only build (no device needed): returns malloc'd arrays, release with ptb_free.  width = 2: ptb_bvh_node
@@ -154,15 +162,16 @@ int ptb_bvh_build_host(const ptb_triangle* tris, int n_tris, const ptb_bvh_param
 
 int ptb_scene_create(ptb_device* dev, const ptb_triangle* tris, int n_tris, const ptb_material* mats, int n_mats,
                      const ptb_bvh_params* bvh_params /* NULL = default */, ptb_scene** out);
-/* same, but the BVH is built ON the device (Morton-order LBVH, csrc/lbvh.cuh): milliseconds for millions of
- * triangles instead of seconds; lower tree quality than the host SAH build.  Needs >= 2 triangles.          */
+/* same, but the BVH is built ON the device: milliseconds for millions of triangles instead of seconds.  By default the
+ * Morton-order LBVH (csrc/lbvh.cuh), of lower tree quality than the host SAH build; bvh_params->builder = PTB_BUILDER_SAH builds
+ * the host's SAH tree instead.  Needs >= 2 triangles.                                                                        */
 int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, int n_tris, const ptb_material* mats, int n_mats,
                          const ptb_bvh_params* bvh_params /* NULL = default */, ptb_scene** out);
 /* The same scene from records that already live on the device (triangles a torch pipeline made or deformed): tris holds n_tris
  * ptb_triangle and mats n_mats ptb_material records (64 bytes each, 16-byte aligned; a ptb_buffer_create buffer or a tensor's
  * storage through ptb_buffer_wrap, both of `dev`).  The tree, node bytes, tri_order, quantised nodes, grid, ptb_scene_info and
- * every render, intersect and shade result equal ptb_scene_create_gpu's for the same records.  bvh_params: max_leaf and pad_rel
- * apply; force_width must be 0 or 2 (the FLAT and 4-wide forms need the host builder).  Needs 2 <= n_tris < 2^28 and
+ * every render, intersect and shade result equal ptb_scene_create_gpu's for the same records.  bvh_params: builder selects the
+ * tree (see ptb_bvh_params); force_width must be 0 or 2 (the FLAT and 4-wide forms need the host builder).  Needs 2 <= n_tris < 2^28 and
  * n_mats >= 1.  The records are checked on the device as ptb_scene_create_gpu checks them on the host (every id in
  * [0, n_mats); every vertex float, w included, |v| <= 3e38), and the message names the lowest offending triangle.  Read on
  * the device's stream, so a device made with ptb_device_create_on_stream on torch's current stream sees the work that wrote

@@ -18,6 +18,7 @@ ACCUM_REFERENCE, ACCUM_LINEAR = 0, 1
 OUTPUT_FLOAT4, OUTPUT_RGB8 = 0, 1
 INTEGRATOR_AUTO, INTEGRATOR_MEGAKERNEL, INTEGRATOR_WAVEFRONT = 0, 1, 2
 ACCEL_BVH, ACCEL_BRUTE = 0, 1
+BUILDER_LBVH, BUILDER_SAH = 0, 1  # ptb_bvh_params.builder: the tree Device.scene(..., gpu_build=True) and scene_from_device build
 
 TRIANGLE_DTYPE = np.dtype(
     [("p1", "<f4", 4), ("p2", "<f4", 4), ("p3", "<f4", 4), ("id", "<i4"), ("padding", "u1", 12)]
@@ -83,7 +84,7 @@ class Counters(C.Structure):
 
 class BvhParams(C.Structure):
     _fields_ = [("max_leaf", C.c_int32), ("pad_rel", C.c_float), ("n_bins", C.c_int32), ("smem_nodes", C.c_int32),
-                ("traverse_cost", C.c_float), ("force_width", C.c_int32), ("reserved", C.c_int32 * 2)]
+                ("traverse_cost", C.c_float), ("force_width", C.c_int32), ("builder", C.c_int32), ("reserved", C.c_int32 * 1)]
 
 
 class Int4(C.Structure):

@@ -16,6 +16,7 @@
 #include "pt_kernels.cuh"
 #include "pt_wavefront.cuh"
 #include "lbvh.cuh"
+#include "sah_build.cuh"
 
 namespace ptb {
 
@@ -507,6 +508,13 @@ extern "C" int ptb_scene_create(ptb_device* dev, const ptb_triangle* tris, int n
     return scene_create_impl(dev, tris, n_tris, mats, n_mats, bvh_params, nullptr, out);
 }
 
+static int check_builder(const char* what, const ptb_bvh_params& bp) {
+    if (bp.builder != PTB_BUILDER_LBVH && bp.builder != PTB_BUILDER_SAH)
+        return fail(PTB_E_INVALID, "%s: builder = %d; PTB_BUILDER_LBVH (0) and PTB_BUILDER_SAH (1) are built on the device", what,
+                    bp.builder);
+    return PTB_OK;
+}
+
 static int check_pad_rel(const char* what, const ptb_bvh_params& bp) {
     if (!(bp.pad_rel > 0.0f) || std::isinf(bp.pad_rel))
         return fail(PTB_E_INVALID, "%s: pad_rel must be a finite number > 0, got %g (without a pad, rounding in "
@@ -514,13 +522,14 @@ static int check_pad_rel(const char* what, const ptb_bvh_params& bp) {
     return PTB_OK;
 }
 
-// The device half of both LBVH constructors (lbvh.cuh).  From n_tris caller-order triangle and n_mats material records on the
-// device (read on dev->stream and not kept): the validation verdicts, the caller-order edge triangles, the packed materials,
-// the light table, the tree and its quantised encoding.  The verdicts and the light table come back in the synchronisation
-// that fetches the tree depth; records that fail validation leave no scene.  Only the root is guaranteed to sit at index 0, so
-// one node is staged in shared memory; everything else is traversed from L2/HBM.
-static int scene_create_lbvh(ptb_device* dev, const char* what, const ptb_triangle* d_tris, int n_tris, const ptb_material* d_mats,
-                             int n_mats, const ptb_bvh_params& bp, ptb_scene** out) {
+// The device half of both device constructors.  From n_tris caller-order triangle and n_mats material records on the device
+// (read on dev->stream and not kept): the validation verdicts, the caller-order edge triangles, the packed materials, the light
+// table, the tree (bp.builder: the LBVH of lbvh.cuh or the host's SAH tree from sah_build.cuh) and its quantised encoding.  The
+// verdicts and the light table come back in the build's last synchronisation; records that fail validation leave no scene.  Of
+// an LBVH only the root is guaranteed to sit at index 0, so one node is staged in shared memory; an SAH tree has the host's
+// breadth-first prefix of smem_nodes nodes.
+static int scene_create_device(ptb_device* dev, const char* what, const ptb_triangle* d_tris, int n_tris, const ptb_material* d_mats,
+                               int n_mats, const ptb_bvh_params& bp, ptb_scene** out) {
     ptb_scene* s = new ptb_scene();
     s->dev = dev; s->n_tris = n_tris; s->n_mats = n_mats;
     s->host_copy_valid = false;
@@ -540,9 +549,14 @@ static int scene_create_lbvh(ptb_device* dev, const char* what, const ptb_triang
     ptd::k_scene_mats<<<grid_m, 256, 0, dev->stream>>>(d_mats, n_mats, s->d_mats);
     ptd::k_scene_lights<<<grid_m, 256, 0, dev->stream>>>(d_tris, n_tris, n_mats, d_lights);
     if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) return fail_out(fail(PTB_E_CUDA, "%s: launch failed: %s", what, cudaGetErrorString(e)));
-    if (int rc = ptd::build_lbvh_device(dev->stream, d_tris, n_tris, bp.max_leaf, bp.pad_rel, &s->d_nodes, &s->d_tris, &s->d_order, &s->depth,
-                                        d_check, check.data(), check.size()))
+    if (bp.builder == PTB_BUILDER_SAH) {
+        if (int rc = ptd::build_sah_device(dev->stream, d_tris, n_tris, bp, &s->d_nodes, &s->d_tris, &s->d_order, &s->n_nodes, &s->depth,
+                                           &s->bfs_nodes, d_check, check.data(), check.size()))
+            return fail_out(rc);
+    } else if (int rc = ptd::build_lbvh_device(dev->stream, d_tris, n_tris, bp.max_leaf, bp.pad_rel, &s->d_nodes, &s->d_tris, &s->d_order,
+                                               &s->depth, d_check, check.data(), check.size())) {
         return fail_out(rc);
+    }
     unsigned long long bad[2];
     std::memcpy(bad, check.data(), sizeof bad);
     if (bad[0] != ~0ull || bad[1] != ~0ull) {  // the lowest offending index; on a tie the id is reported, as the host loop does
@@ -578,6 +592,7 @@ extern "C" int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, i
     ptb_bvh_params bp;
     if (bvh_params) bp = *bvh_params; else ptb_bvh_params_default(&bp);
     if (int rc = check_pad_rel("ptb_scene_create_gpu", bp)) return rc;
+    if (int rc = check_builder("ptb_scene_create_gpu", bp)) return rc;
     if (set_device(dev)) return PTB_E_CUDA;
     ptb_triangle* d_raw = nullptr;  // the triangle records, then the material records
     if (cudaMalloc((void**)&d_raw, (size_t(n_tris) + size_t(n_mats)) * 64) != cudaSuccess)
@@ -589,7 +604,7 @@ extern "C" int ptb_scene_create_gpu(ptb_device* dev, const ptb_triangle* tris, i
         cudaStreamSynchronize(dev->stream);
         rc = fail(PTB_E_CUDA, "ptb_scene_create_gpu: upload failed");
     } else {
-        rc = scene_create_lbvh(dev, "ptb_scene_create_gpu", d_raw, n_tris, d_rawm, n_mats, bp, out);
+        rc = scene_create_device(dev, "ptb_scene_create_gpu", d_raw, n_tris, d_rawm, n_mats, bp, out);
     }
     cudaFree(d_raw);
     return rc;
@@ -616,9 +631,10 @@ extern "C" int ptb_scene_create_from_device(ptb_device* dev, ptb_buffer* tris, i
     if (bp.force_width != 0 && bp.force_width != 2)
         return fail(PTB_E_INVALID, "ptb_scene_create_from_device: force_width = %d; only the binary form (0 or 2) is built on the device",
                     bp.force_width);
+    if (int rc = check_builder("ptb_scene_create_from_device", bp)) return rc;
     if (set_device(dev)) return PTB_E_CUDA;
-    return scene_create_lbvh(dev, "ptb_scene_create_from_device", static_cast<const ptb_triangle*>(tris->d_ptr), n_tris,
-                             static_cast<const ptb_material*>(mats->d_ptr), n_mats, bp, out);
+    return scene_create_device(dev, "ptb_scene_create_from_device", static_cast<const ptb_triangle*>(tris->d_ptr), n_tris,
+                               static_cast<const ptb_material*>(mats->d_ptr), n_mats, bp, out);
 }
 
 extern "C" int ptb_bvh_build_host(const ptb_triangle* tris, int n_tris, const ptb_bvh_params* bvh_params, int width,
